@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the CGVAE equivariant message-passing hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl cuda|reference] [--workload c2_chignolin|c1_dipeptide]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], the configuration the metric is quoted on): chignolin all-atom CGVAE,
 175 atoms, n_cgs 6, batch 2, enc_nconv 2 / dec_nconv 9, n_basis 600, n_rbf 10, cutoffs 12 / 25 A, synthetic
@@ -20,6 +21,11 @@ sample (the oracle port only if the reference install is missing).
 
 --impl reference: times the unmodified reference's own training step (its CPU PyTorch path, all host threads) for the
 same metric / config; under torchrun only rank 0 runs and prints.
+
+--dump-outputs DIR (--impl cuda): after the K timed steps, rank 0 writes what the last of them computed as float32 .npy
+files: `loss` (the value the step returns), `parameters` (the used parameters after its Adam update) and `gradients` (the
+gradients it formed), the two buffers in flat-buffer order and, above 4 Mi floats, sampled at the same seeded positions on
+every run.  Inputs, weights and noise are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -61,7 +67,13 @@ def _args():
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of one CUDA graph per step")
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary workloads (c3 sampling, c4 protein, c5 layer)")
     ap.add_argument("--fixed-eps", action="store_true", help="pass a fixed noise tensor instead of drawing it inside the step")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs applies to --impl cuda")
+    return args
 
 
 def _peaks():
@@ -349,6 +361,27 @@ def _timeit(fn, warm, iters):
     return e0.elapsed_time(e1) / iters
 
 
+DUMP_SAMPLE = 1 << 22          # floats kept per buffer: 2 x 16 MB at most
+
+
+def _dump_outputs(out_dir, loss, trainer):
+    """loss / parameters / gradients of the step that just ran as float32 DIR/<name>.npy (see --dump-outputs).  The sample
+    positions depend only on the buffer length (fixed seed), so runs of the same workload keep the same elements."""
+    import numpy as np
+    import torch
+    params = torch.cat([p.detach().reshape(-1) for p in trainer.flat.params])
+    grads = trainer.flat.flat
+    idx = None
+    if params.numel() > DUMP_SAMPLE:
+        pick = np.random.default_rng(0).choice(params.numel(), DUMP_SAMPLE, replace=False)
+        idx = torch.from_numpy(np.sort(pick)).to(params.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", loss.detach().reshape(-1)), ("parameters", params), ("gradients", grads)):
+        if idx is not None and name != "loss":
+            t = t[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.to(torch.float32).cpu().numpy())
+
+
 def _extra_c3(dev, world, rank):
     """BASELINE config 3: chignolin sampling, n_ensemble 8 -- the prior once + 8 decoder passes per conformation as ONE CUDA
     graph replay (train.GraphedSampler); under torchrun the 8 members are sharded over the ranks and all-gathered."""
@@ -535,11 +568,13 @@ def run_cuda(args, cfg):
     sync_all()
     e0.record()
     for i in range(args.steps):
-        run_step(i % args.pool)
+        step_loss = run_step(i % args.pool)
     e1.record()
     sync_all()
     launches = (graphed.launches_per_step * args.steps) if use_graph else (ops.launch_count() - launches0)
     clock_info = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, step_loss, trainer)
     ms_total = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms_total, op=dist.ReduceOp.MAX)
