@@ -431,7 +431,26 @@ def gemm(form, A, B, M, N, K, bias=None, act=0, z_out=False, z_in=None, dact=0, 
                            % (A.dtype, tuple(A.stride()), B.dtype, tuple(B.stride())))
     lib = _lib.load()
     dev = A.device
+    if out is not None and (out.dtype != torch.float32 or out.device != dev or tuple(out.shape) != (M, N)
+                            or (N > 1 and out.stride(1) != 1)):
+        raise RuntimeError("gemm: out must be a float32 (%d, %d) tensor with unit inner stride on %s (got %s %s %s on %s)"
+                           % (M, N, dev, out.dtype, tuple(out.shape), tuple(out.stride()), out.device))
     C = out if out is not None else torch.empty((M, N), dtype=torch.float32, device=dev)
+    # the kernels read bias[n] and z_in / add / z_out at m * ldc + n, with ldc = C's row stride
+    ldc = C.stride(0)
+    if bias is not None and (bias.dtype != torch.float32 or bias.dim() != 1 or bias.numel() != N
+                             or not bias.is_contiguous() or bias.device != dev):
+        raise RuntimeError("gemm: bias must be a contiguous float32 vector of length %d on %s (got %s %s %s on %s)"
+                           % (N, dev, bias.dtype, tuple(bias.shape), tuple(bias.stride()), bias.device))
+    for name, t in (("z_in", z_in), ("add", add)):
+        if t is not None and (t.dtype != torch.float32 or tuple(t.shape) != (M, N) or (N > 1 and t.stride(1) != 1)
+                              or (M > 1 and t.stride(0) != ldc) or t.device != dev):
+            raise RuntimeError("gemm: %s must be a float32 (%d, %d) tensor on %s with the row stride of the output (%d) "
+                               "and unit inner stride (got %s %s %s on %s)"
+                               % (name, M, N, dev, ldc, t.dtype, tuple(t.shape), tuple(t.stride()), t.device))
+    if z_out and M > 1 and ldc != N:
+        raise RuntimeError("gemm: z_out=True needs an output with row stride %d (the pre-activation copy is a contiguous "
+                           "(M, N) tensor indexed with the output's row stride); got row stride %d" % (N, ldc))
     Z = torch.empty((M, N), dtype=torch.float32, device=dev) if z_out else None
     tiles = ((M + 63) // 64) * ((N + 63) // 64) if M > 32 else ((N + 31) // 32)
     st = _stream()
@@ -440,7 +459,7 @@ def gemm(form, A, B, M, N, K, bias=None, act=0, z_out=False, z_in=None, dact=0, 
         ws = torch.empty(_SPLITK_WS_BYTES, dtype=torch.uint8, device=dev)
         tk = _tickets(dev, st)
     t0 = TIMER.begin("gemm") if TIMER is not None else None
-    _lib.check(lib.cgvae_gemm(form, _p(A), A.stride(0), _p(B), B.stride(0), _p(C), C.stride(0), M, N, K, _p(bias), act, _p(Z),
+    _lib.check(lib.cgvae_gemm(form, _p(A), A.stride(0), _p(B), B.stride(0), _p(C), ldc, M, N, K, _p(bias), act, _p(Z),
                               _p(z_in), dact, _p(add), _p(ws), _SPLITK_WS_BYTES if ws is not None else 0, _p(tk),
                               _N_TICKETS if tk is not None else 0, st), "gemm")
     if t0 is not None:
@@ -625,8 +644,10 @@ def linear_bwd_weight(gy, x, param=None, shape=None):
 
 def colsum(X, param=None):
     _need_cuda(X)
-    lib = _lib.load()
     M, N = X.shape
+    if X.dtype != torch.float32 or (N > 1 and X.stride(1) != 1):     # the kernels read X[m * ldx + n]
+        raise RuntimeError("colsum: X must be float32 with unit inner stride (got %s %s)" % (X.dtype, tuple(X.stride())))
+    lib = _lib.load()
     out = _grad_out(param, (N,)) if param is not None else torch.empty(N, dtype=torch.float32, device=X.device)
     if deferring(M) and _has_sink(param) and X.stride(1) == 1:
         _DEFERRED.append((X, None, None, out.detach()))
