@@ -12,5 +12,6 @@ from .conv import (ContractiveMessageBlock, EquiMessageBlock, EquiMessageCross, 
 from .data import (CG_collate, CGDataset, DeviceCGDataset, batch_to, get_neighbor_list,  # noqa: F401
                    get_neighbor_list_batch)
 from .modules import Dense, DistanceEmbed, make_directed  # noqa: F401
+from .ops import get_matmul_precision, matmul_precision, set_matmul_precision  # noqa: F401
 
 __version__ = "0.1.0"

@@ -72,6 +72,8 @@ SIGNATURES = {
     "cgvae_bond_graph": (_INT, [_P, _P, _I64, _F32, _P, _P]),
     "cgvae_sample_quality": (_INT, [_P, _P, _P, _P, _I64, _I64, _F32, _P, _P, _P]),
     "cgvae_set_pdl": (_INT, [_INT]),
+    "cgvae_set_matmul_precision": (_INT, [_INT]),
+    "cgvae_get_matmul_precision": (_INT, []),
     "cgvae_register_const_range": (_INT, [_P, _SZ]),
     "cgvae_grad_sumsq": (_INT, [_P, _I64, _P, _P, _SZ, _P]),
     "cgvae_adam_apply": (_INT, [_P, _P, _P, _P, _I64, _F32, _F32, _F32, _F32, _F32, _F32, _P, _P, _INT, _F32, _F32, _P, _P, _SZ, _P]),

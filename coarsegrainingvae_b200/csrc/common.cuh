@@ -76,6 +76,8 @@ __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.lau
   } while (0)
 
 bool pdl_enabled();
+// 0: the tensor-core GEMMs and the message filter run 3xTF32 (fp32 parity); 1: 1xTF32 (graph.cu, cgvae_set_matmul_precision)
+int matmul_precision();
 // inside a parameter range registered with cgvae_register_const_range, and PDL on (gemm_stream.cu)
 bool weights_are_constant(const void* p, size_t bytes);
 

@@ -50,7 +50,6 @@ constexpr uint32_t TMEM_COLS = 512;
 static_assert((1 + NBIG) * BN <= (int)TMEM_COLS, "accumulators must fit in TMEM");
 constexpr int PS = BN + 4;                                             // row stride (floats) of a parked partial tile
 constexpr int MAX_KT_PER_CTA = 96;   // longest accumulation chain per CTA (k-steps of 32): keeps the 1e-5 gate with margin
-static_assert(BM * PS * 4 <= STAGES * STAGE_BYTES, "partial tile must fit in the pipeline stages");
 
 struct Ep {
   const float* bias;
@@ -235,11 +234,81 @@ __device__ __forceinline__ void load_acc(uint32_t taddr, int nbig, float (&out)[
   }
 }
 
-template <bool A_KC, bool B_KC>
-__global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a,
-                                                                 const __grid_constant__ CUtensorMap map_b, float* __restrict__ C,
-                                                                 int64_t ldc, int64_t M, int64_t N, int64_t K, int kt_per_split, Ep ep,
-                                                                 int split_mode, int cluster_size, float* __restrict__ partial, int b_const) {
+// ONE = false: 3xTF32 (the default).  ONE = true: 1xTF32 (cgvae_set_matmul_precision(1)) -- the stage holds the raw tile
+// only, rounded to nearest TF32 in place by the split warps, so twice as many stages fit in the same shared memory, and
+// one MMA per K = 8 accumulates into a single accumulator (its truncation drift, <= chain length x 2^-23 relative, is
+// negligible next to the 2^-11 of the operand rounding).
+template <bool ONE>
+struct Ring {
+  static constexpr int STAGES = ONE ? 2 * tc::STAGES : tc::STAGES;
+  static constexpr uint32_t STAGE_BYTES = ONE ? RAW_BYTES : tc::STAGE_BYTES;
+  static_assert(STAGES * STAGE_BYTES == tc::STAGES * tc::STAGE_BYTES, "both forms use the same shared memory");
+    static_assert(3 * STAGES * 8 + 4 * 8 + 4 <= (int)BAR_BYTES, "barriers must fit in BAR_BYTES");
+};
+
+// the split warps' pass over one landed stage: 3xTF32 writes the lo tile next to the raw one; 1xTF32 rounds the raw tile
+// to nearest TF32 in place (the tensor core would truncate: a one-sided error that grows with K instead of averaging out)
+template <bool ONE, int NT>
+__device__ __forceinline__ void split_stage(char* stage, int t, int split_mode) {
+  const float4* raw = reinterpret_cast<const float4*>(stage);
+  constexpr int PER = (int)(RAW_BYTES / 16) / NT;   // 8 float4 per thread
+  float4 x[PER];
+#pragma unroll
+  for (int it = 0; it < PER; ++it) x[it] = raw[t + it * NT];
+  if constexpr (ONE) {
+    float4* rawm = reinterpret_cast<float4*>(stage);
+#pragma unroll
+    for (int it = 0; it < PER; ++it)
+      rawm[t + it * NT] = make_float4(to_tf32(x[it].x), to_tf32(x[it].y), to_tf32(x[it].z), to_tf32(x[it].w));
+  } else {
+    float4* lo = reinterpret_cast<float4*>(stage + RAW_BYTES);
+    if (split_mode == 0) {
+#pragma unroll
+      for (int it = 0; it < PER; ++it) {
+        float4 l;
+        l.x = lo_of(x[it].x);
+        l.y = lo_of(x[it].y);
+        l.z = lo_of(x[it].z);
+        l.w = lo_of(x[it].w);
+        lo[t + it * NT] = l;
+      }
+    } else {
+      // round-to-nearest hi written back over the raw tile: |lo| <= 2^-12 |x| keeps one more bit than the truncating split
+      float4* rawm = reinterpret_cast<float4*>(stage);
+#pragma unroll
+      for (int it = 0; it < PER; ++it) {
+        float4 h, l;
+        split_tf32(x[it].x, h.x, l.x);
+        split_tf32(x[it].y, h.y, l.y);
+        split_tf32(x[it].z, h.z, l.z);
+        split_tf32(x[it].w, h.w, l.w);
+        rawm[t + it * NT] = h;
+        lo[t + it * NT] = l;
+      }
+    }
+  }
+}
+
+// 32 columns of the single 1xTF32 accumulator for this thread's row
+__device__ __forceinline__ void load_acc1(uint32_t taddr, bool any, float (&out)[32]) {
+  if (!any) {                            // empty K-slice
+#pragma unroll
+    for (int j = 0; j < 32; ++j) out[j] = 0.f;
+    return;
+  }
+  uint32_t r[32];
+  tmem_ld32(taddr, r);
+  tmem_wait_ld();
+#pragma unroll
+  for (int j = 0; j < 32; ++j) out[j] = __uint_as_float(r[j]);
+}
+
+template <bool A_KC, bool B_KC, bool ONE>
+__device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUtensorMap& map_b, float* __restrict__ C, int64_t ldc,
+                                             int64_t M, int64_t N, int64_t K, int kt_per_split, const Ep& ep, int split_mode,
+                                             int cluster_size, float* __restrict__ partial, int b_const) {
+  constexpr int STAGES = Ring<ONE>::STAGES;
+  constexpr uint32_t STAGE_BYTES = Ring<ONE>::STAGE_BYTES;
   // b_const: B is a weight matrix inside a registered parameter range -- the producer issues its first tiles BEFORE the
   // dependency wait of the programmatic dependent launch (they overlap with the preceding kernel), A follows the wait
   if (!b_const) CGVAE_KERNEL_PROLOGUE();
@@ -307,36 +376,7 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_co
     for (int i = 0; i < nkt; ++i) {
       const int s = i % STAGES;
       mbar_wait(&raw_full[s], (uint32_t)(i / STAGES) & 1u);
-      const float4* raw = reinterpret_cast<const float4*>(smem + (uint32_t)s * STAGE_BYTES);
-      float4* lo = reinterpret_cast<float4*>(smem + (uint32_t)s * STAGE_BYTES + RAW_BYTES);
-      constexpr int PER = (int)(RAW_BYTES / 16) / (NUM_SPLIT_WARPS * 32);   // 8 float4 per thread
-      float4 x[PER];
-#pragma unroll
-      for (int it = 0; it < PER; ++it) x[it] = raw[tid + it * NUM_SPLIT_WARPS * 32];
-      if (split_mode == 0) {
-#pragma unroll
-        for (int it = 0; it < PER; ++it) {
-          float4 l;
-          l.x = lo_of(x[it].x);
-          l.y = lo_of(x[it].y);
-          l.z = lo_of(x[it].z);
-          l.w = lo_of(x[it].w);
-          lo[tid + it * NUM_SPLIT_WARPS * 32] = l;
-        }
-      } else {
-        // round-to-nearest hi written back over the raw tile: |lo| <= 2^-12 |x| keeps one more bit than the truncating split
-        float4* rawm = const_cast<float4*>(raw);
-#pragma unroll
-        for (int it = 0; it < PER; ++it) {
-          float4 h, l;
-          split_tf32(x[it].x, h.x, l.x);
-          split_tf32(x[it].y, h.y, l.y);
-          split_tf32(x[it].z, h.z, l.z);
-          split_tf32(x[it].w, h.w, l.w);
-          rawm[tid + it * NUM_SPLIT_WARPS * 32] = h;
-          lo[tid + it * NUM_SPLIT_WARPS * 32] = l;
-        }
-      }
+      split_stage<ONE, NUM_SPLIT_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, tid, split_mode);
       fence_async_smem();            // generic-proxy writes -> visible to the tensor core (async proxy)
       __syncwarp();
       if (lane == 0) mbar_arrive(&lo_done[s]);
@@ -381,11 +421,15 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_co
 #pragma unroll
         for (int ks = 0; ks < BK / 8; ++ks) {
           const uint32_t ao = (uint32_t)ks * a_step, bo = (uint32_t)ks * b_step;
-          const uint32_t d_big = tmem_base + (uint32_t)(1 + i % NBIG) * BN;
-          umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_hi + bo), (i > 0 || ks > 0) ? 1u : 0u, idesc);
-          umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
-          if (split_mode == 2) umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
-          umma_tf32_ss(d_big, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), (i >= NBIG || ks > 0) ? 1u : 0u, idesc);
+          if constexpr (ONE) {
+            umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), (i > 0 || ks > 0) ? 1u : 0u, idesc);
+          } else {
+            const uint32_t d_big = tmem_base + (uint32_t)(1 + i % NBIG) * BN;
+            umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_hi + bo), (i > 0 || ks > 0) ? 1u : 0u, idesc);
+            umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
+            if (split_mode == 2) umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
+            umma_tf32_ss(d_big, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), (i >= NBIG || ks > 0) ? 1u : 0u, idesc);
+          }
         }
         umma_commit(&empty_bar[s]);                  // stage reusable once these MMAs have read it
         if (i == nkt - 1) umma_commit(acc_bar);      // accumulator complete
@@ -410,7 +454,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_co
       for (int cb = 0; cb < BN / 64; ++cb) {
         const int c0 = half * (BN / 2) + cb * 32;
         float r[32];
-        load_acc(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, min(nkt, NBIG), r);
+        if constexpr (ONE) load_acc1(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, nkt > 0, r);
+        else load_acc(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, min(nkt, NBIG), r);
 #pragma unroll
         for (int j = 0; j < 32; ++j) tr[lane * 33 + j] = r[j];   // row = lane, column = j
         __syncwarp();
@@ -431,7 +476,8 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_co
       for (int cb = 0; cb < BN / 64; ++cb) {
         const int c0 = half * (BN / 2) + cb * 32;
         float r[32];
-        load_acc(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, min(nkt, NBIG), r);
+        if constexpr (ONE) load_acc1(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, nkt > 0, r);
+        else load_acc(tmem_base + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, min(nkt, NBIG), r);
 #pragma unroll
         for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(P + row * PS + c0 + j) = make_float4(r[j], r[j + 1], r[j + 2], r[j + 3]);
       }
@@ -457,6 +503,20 @@ __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(const __grid_co
   }
 }
 
+#define GEMM_TC_PARAMS                                                                                                          \
+  const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, float* __restrict__ C, int64_t ldc,    \
+      int64_t M, int64_t N, int64_t K, int kt_per_split, Ep ep, int split_mode, int cluster_size, float* __restrict__ partial, \
+      int b_const
+template <bool A_KC, bool B_KC>
+__global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(GEMM_TC_PARAMS) {
+  gemm_tc_body<A_KC, B_KC, false>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, split_mode, cluster_size, partial, b_const);
+}
+template <bool A_KC, bool B_KC>
+__global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc1_kernel(GEMM_TC_PARAMS) {
+  gemm_tc_body<A_KC, B_KC, true>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, split_mode, cluster_size, partial, b_const);
+}
+#undef GEMM_TC_PARAMS
+
 
 // ---------------------------------------------------------------------------------------------------------------------------
 // Persistent variant for problems with many output tiles and a short k-loop (the 16 000 .. 128 000-row layers of the protein
@@ -472,11 +532,12 @@ constexpr uint32_t P_SCRATCH_BYTES = P_EPI_WARPS * 32 * 33 * 4;
 constexpr uint32_t P_SMEM_BYTES = STAGES * STAGE_BYTES + P_SCRATCH_BYTES + BAR_BYTES + 1024;
 constexpr int P_MAX_KT = 40;          // one big accumulator per tile: chain length bounded like the round-1 kernel (K <= 1280)
 
-template <bool A_KC, bool B_KC>
-__global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const __grid_constant__ CUtensorMap map_a,
-                                                                          const __grid_constant__ CUtensorMap map_b, float* __restrict__ C,
-                                                                          int64_t ldc, int64_t M, int64_t N, int64_t K, Ep ep,
-                                                                          int tiles_n, int n_tiles) {
+template <bool A_KC, bool B_KC, bool ONE>
+__device__ __forceinline__ void gemm_tc_persistent_body(const CUtensorMap& map_a, const CUtensorMap& map_b, float* __restrict__ C,
+                                                        int64_t ldc, int64_t M, int64_t N, int64_t K, const Ep& ep, int tiles_n,
+                                                        int n_tiles) {
+  constexpr int STAGES = Ring<ONE>::STAGES;
+  constexpr uint32_t STAGE_BYTES = Ring<ONE>::STAGE_BYTES;
   CGVAE_KERNEL_PROLOGUE();
   extern __shared__ __align__(1024) char smem_raw[];
   char* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -559,9 +620,13 @@ __global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const 
           for (int ks = 0; ks < BK / 8; ++ks) {
             const uint32_t ao = (uint32_t)ks * a_step, bo = (uint32_t)ks * b_step;
             const uint32_t acc = (kt > 0 || ks > 0) ? 1u : 0u;
-            umma_tf32_ss(d_small, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_hi + bo), acc, idesc);
-            umma_tf32_ss(d_small, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
-            umma_tf32_ss(d_big, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), acc, idesc);
+            if constexpr (ONE) {
+              umma_tf32_ss(d_small, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), acc, idesc);   // one accumulator
+            } else {
+              umma_tf32_ss(d_small, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_hi + bo), acc, idesc);
+              umma_tf32_ss(d_small, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
+              umma_tf32_ss(d_big, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), acc, idesc);
+            }
           }
           umma_commit(&empty_bar[s]);
           if (kt == num_kt - 1) umma_commit(&acc_full[buf]);
@@ -585,7 +650,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const 
       for (int cb = 0; cb < BN / 32; ++cb) {
         uint32_t r[32], t[32];
         tmem_ld32(t_small + (uint32_t)cb * 32u, r);
-        tmem_ld32(t_small + BN + (uint32_t)cb * 32u, t);
+        if constexpr (!ONE) tmem_ld32(t_small + BN + (uint32_t)cb * 32u, t);
         tmem_wait_ld();
         if (cb == BN / 32 - 1) {                              // everything of this set is in registers: hand it back
           tc_fence_before();
@@ -593,7 +658,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const 
           if (lane == 0) mbar_arrive(&acc_empty[buf]);
         }
 #pragma unroll
-        for (int j = 0; j < 32; ++j) tr[lane * 33 + j] = __uint_as_float(r[j]) + __uint_as_float(t[j]);
+        for (int j = 0; j < 32; ++j) tr[lane * 33 + j] = ONE ? __uint_as_float(r[j]) : __uint_as_float(r[j]) + __uint_as_float(t[j]);
         __syncwarp();
         if (m0 + 32 * q < M) store_block(mode, ep, tr, lane, C, ldc, m0 + 32 * q, n0 + cb * 32 + lane, M, N);
         __syncwarp();
@@ -607,21 +672,7 @@ __global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const 
       for (int kt = 0; kt < num_kt; ++kt, ++it) {
         const int s = it % STAGES;
         mbar_wait(&raw_full[s], (uint32_t)(it / STAGES) & 1u);
-        const float4* raw = reinterpret_cast<const float4*>(smem + (uint32_t)s * STAGE_BYTES);
-        float4* lo = reinterpret_cast<float4*>(smem + (uint32_t)s * STAGE_BYTES + RAW_BYTES);
-        constexpr int PER = (int)(RAW_BYTES / 16) / (P_LO_WARPS * 32);
-        float4 x[PER];
-#pragma unroll
-        for (int i = 0; i < PER; ++i) x[i] = raw[t0 + i * P_LO_WARPS * 32];
-#pragma unroll
-        for (int i = 0; i < PER; ++i) {
-          float4 l;
-          l.x = lo_of(x[i].x);
-          l.y = lo_of(x[i].y);
-          l.z = lo_of(x[i].z);
-          l.w = lo_of(x[i].w);
-          lo[t0 + i * P_LO_WARPS * 32] = l;
-        }
+        split_stage<ONE, P_LO_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, t0, 0);
         fence_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive(&lo_done[s]);
@@ -635,6 +686,19 @@ __global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(const 
     tmem_dealloc<TMEM_COLS>(tmem_base);
   }
 }
+
+#define GEMM_TC_P_PARAMS                                                                                                        \
+  const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, float* __restrict__ C, int64_t ldc,    \
+      int64_t M, int64_t N, int64_t K, Ep ep, int tiles_n, int n_tiles
+template <bool A_KC, bool B_KC>
+__global__ void __launch_bounds__(P_THREADS, 1) gemm_tc_persistent_kernel(GEMM_TC_P_PARAMS) {
+  gemm_tc_persistent_body<A_KC, B_KC, false>(map_a, map_b, C, ldc, M, N, K, ep, tiles_n, n_tiles);
+}
+template <bool A_KC, bool B_KC>
+__global__ void __launch_bounds__(P_THREADS, 1) gemm_tc1_persistent_kernel(GEMM_TC_P_PARAMS) {
+  gemm_tc_persistent_body<A_KC, B_KC, true>(map_a, map_b, C, ldc, M, N, K, ep, tiles_n, n_tiles);
+}
+#undef GEMM_TC_P_PARAMS
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
@@ -711,6 +775,8 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
   const int b_const = (form != CGVAE_GEMM_TN &&
                        weights_are_constant(B, sizeof(float) * (size_t)(((b_kc ? N : K) - 1) * ldb + (b_kc ? K : N)))) ? 1 : 0;
   tc::Ep ep{bias, act, z_out, z_in, dact, add};
+  // the precision mode picks the kernel only: S, groups, persistent eligibility and grid are those of the 3xTF32 kernels
+  const bool one = matmul_precision() == 1;
   static const bool persistent_on = [] { const char* e = getenv("CGVAE_TC_PERSISTENT"); return !(e && e[0] == '0'); }();
   if (persistent_on && S == 1 && groups == 1 && tiles >= 2 * kNumSM && num_kt <= tc::P_MAX_KT) {
     cudaLaunchConfig_t pc = {};
@@ -724,7 +790,7 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
     pc.attrs = pattr;
     pc.numAttrs = pdl_enabled() ? 1 : 0;
     const int tiles_n = (int)ceil_div(N, tc::BN), n_tiles = (int)tiles;
-    static bool p_attr_done[3] = {false, false, false};
+    static bool p_attr_done[6] = {false, false, false, false, false, false};
     auto pgo = [&](auto kernel, int idx) {
       if (!p_attr_done[idx]) {
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::P_SMEM_BYTES);
@@ -732,9 +798,15 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
       }
       (void)cudaLaunchKernelEx(&pc, kernel, map_a, map_b, C, ldc, M, N, K, ep, tiles_n, n_tiles);
     };
-    if (a_kc && b_kc) pgo(tc::gemm_tc_persistent_kernel<true, true>, 0);
-    else if (a_kc) pgo(tc::gemm_tc_persistent_kernel<true, false>, 1);
-    else pgo(tc::gemm_tc_persistent_kernel<false, false>, 2);
+    if (one) {
+      if (a_kc && b_kc) pgo(tc::gemm_tc1_persistent_kernel<true, true>, 3);
+      else if (a_kc) pgo(tc::gemm_tc1_persistent_kernel<true, false>, 4);
+      else pgo(tc::gemm_tc1_persistent_kernel<false, false>, 5);
+    } else {
+      if (a_kc && b_kc) pgo(tc::gemm_tc_persistent_kernel<true, true>, 0);
+      else if (a_kc) pgo(tc::gemm_tc_persistent_kernel<true, false>, 1);
+      else pgo(tc::gemm_tc_persistent_kernel<false, false>, 2);
+    }
     return 1;
   }
   if (groups > 1) ep = tc::Ep{nullptr, 0, nullptr, nullptr, 0, nullptr};
@@ -753,7 +825,7 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl_enabled() ? 2 : 1;
-  static bool attr_done[3] = {false, false, false};
+  static bool attr_done[6] = {false, false, false, false, false, false};
   auto go = [&](auto kernel, int idx) {
     if (!attr_done[idx]) {
       cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES);
@@ -761,9 +833,15 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
     }
     (void)cudaLaunchKernelEx(&cfg, kernel, map_a, map_b, C, ldc, M, N, K, kps, ep, split_mode, S, partial, b_const);
   };
-  if (a_kc && b_kc) go(tc::gemm_tc_kernel<true, true>, 0);
-  else if (a_kc) go(tc::gemm_tc_kernel<true, false>, 1);
-  else go(tc::gemm_tc_kernel<false, false>, 2);
+  if (one) {
+    if (a_kc && b_kc) go(tc::gemm_tc1_kernel<true, true>, 3);
+    else if (a_kc) go(tc::gemm_tc1_kernel<true, false>, 4);
+    else go(tc::gemm_tc1_kernel<false, false>, 5);
+  } else {
+    if (a_kc && b_kc) go(tc::gemm_tc_kernel<true, true>, 0);
+    else if (a_kc) go(tc::gemm_tc_kernel<true, false>, 1);
+    else go(tc::gemm_tc_kernel<false, false>, 2);
+  }
   return groups > 1 ? 1 + groups : 1;          // > 1: the caller reduces `groups` partial matrices in ws
 }
 

@@ -25,6 +25,11 @@ bool pdl_enabled() {
   return v != 0;
 }
 
+// Matmul precision of the tensor-core contractions (cgvae_set_matmul_precision): 0 = 3xTF32 (default), 1 = 1xTF32.
+// Read by the dispatchers at every launch; a captured CUDA graph keeps the kernels it was captured with.
+static std::atomic<int> g_matmul_precision{0};
+int matmul_precision() { return g_matmul_precision.load(std::memory_order_relaxed); }
+
 // ------------------------------------------------------------------------------------------
 // scans (single CTA, 1024 threads x 8 items per sweep; inputs here are <= a few 1e5 long)
 // ------------------------------------------------------------------------------------------
@@ -500,6 +505,13 @@ int cgvae_set_pdl(int on) {
   cgvae::g_pdl.store(on ? 1 : 0, std::memory_order_relaxed);
   return prev;
 }
+
+int cgvae_set_matmul_precision(int mode) {
+  CGVAE_REQUIRE(mode == 0 || mode == 1, "set_matmul_precision: mode must be 0 (\"highest\", 3xTF32) or 1 (\"high\", 1xTF32), got %d",
+                mode);
+  return cgvae::g_matmul_precision.exchange(mode, std::memory_order_relaxed);
+}
+int cgvae_get_matmul_precision(void) { return cgvae::matmul_precision(); }
 
 int cgvae_set_error_flags(int device, int32_t* flags) {
   CGVAE_REQUIRE(device >= 0 && device < kMaxDevices, "set_error_flags: bad device %d", device);

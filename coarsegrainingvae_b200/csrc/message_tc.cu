@@ -243,23 +243,29 @@ __device__ __forceinline__ void umma_commit_a(uint32_t bar_addr) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_addr) : "memory");
 }
 
-// filter MMAs of one batch: D_k = A_k[tmem] * B^T[smem] for every split, 3xTF32 (small terms first), K = 16 in two steps
-template <int KS>
+// filter MMAs of one batch: D_k = A_k[tmem] * B^T[smem] for every split, 3xTF32 (small terms first), K = 16 in two steps.
+// ONE (1xTF32, cgvae_set_matmul_precision(1)): the hi * hi product only -- both hi halves are already rounded to nearest
+template <int KS, bool ONE>
 __device__ __forceinline__ void issue_filter_mmas(uint32_t stage_addr, uint32_t tmem_base, uint32_t d_col) {
   constexpr uint32_t idesc = idesc_tf32(128, NB);
   const uint64_t b_hi = make_desc(stage_addr + REC_BHI, kLBO, TILE_SBO);
-  const uint64_t b_lo = b_hi + (uint64_t)((REC_BLO - REC_BHI) >> 4);
+  [[maybe_unused]] const uint64_t b_lo = b_hi + (uint64_t)((REC_BLO - REC_BHI) >> 4);
 #pragma unroll
   for (int k = 0; k < KS; ++k) {
-    const uint32_t a_hi = tmem_base + Cols<KS>::A + (uint32_t)(k * 2 * KT), a_lo = a_hi + KT;
+    const uint32_t a_hi = tmem_base + Cols<KS>::A + (uint32_t)(k * 2 * KT);
+    [[maybe_unused]] const uint32_t a_lo = a_hi + KT;
     const uint32_t d = tmem_base + d_col + (uint32_t)(k * NB);
 #pragma unroll
     for (int ks = 0; ks < KT / 8; ++ks) {
       const uint32_t ao = (uint32_t)ks * 8;
       const uint64_t bo = (uint64_t)((ks * 2 * kLBO) >> 4);
-      umma_tf32_ts(d, a_lo + ao, b_hi + bo, ks > 0 ? 1u : 0u, idesc);
-      umma_tf32_ts(d, a_hi + ao, b_lo + bo, 1u, idesc);
-      umma_tf32_ts(d, a_hi + ao, b_hi + bo, 1u, idesc);
+      if constexpr (ONE) {
+        umma_tf32_ts(d, a_hi + ao, b_hi + bo, ks > 0 ? 1u : 0u, idesc);
+      } else {
+        umma_tf32_ts(d, a_lo + ao, b_hi + bo, ks > 0 ? 1u : 0u, idesc);
+        umma_tf32_ts(d, a_hi + ao, b_lo + bo, 1u, idesc);
+        umma_tf32_ts(d, a_hi + ao, b_hi + bo, 1u, idesc);
+      }
     }
   }
 }
@@ -325,14 +331,19 @@ __device__ __forceinline__ bool next_segment(const int32_t* __restrict__ bptr, i
 // CTA that owns global batch x under the partition lo_b = b * T / G
 __device__ __forceinline__ int cta_of_batch(int64_t x, int64_t T, int G) { return (int)(((x + 1) * G - 1) / T); }
 
-template <int KS, int RC, int NSUB>
-__global__ void __launch_bounds__((4 * NSUB + 2) * 32, 1) message_tc_fwd_kernel(
-    const float* __restrict__ phi, const float* __restrict__ v_send, const float* __restrict__ v_recv,
-    const int32_t* __restrict__ bptr, const int32_t* __restrict__ ngroups, const char* __restrict__ rec,
-    const float* __restrict__ Wf, const float* __restrict__ bf, int64_t n_recv, int F, int R,
-    const float* __restrict__ res_s, const float* __restrict__ res_v, int v_is_zero, float* __restrict__ out_s,
-    float* __restrict__ out_v, float* __restrict__ q_out, int n_chunks, int n_items, int32_t* __restrict__ tickets,
-    float* __restrict__ part_ws) {
+#define MESSAGE_TC_FWD_PARAMS                                                                                              \
+  const float* __restrict__ phi, const float* __restrict__ v_send, const float* __restrict__ v_recv,                        \
+      const int32_t* __restrict__ bptr, const int32_t* __restrict__ ngroups, const char* __restrict__ rec,                  \
+      const float* __restrict__ Wf, const float* __restrict__ bf, int64_t n_recv, int F, int R,                             \
+      const float* __restrict__ res_s, const float* __restrict__ res_v, int v_is_zero, float* __restrict__ out_s,           \
+      float* __restrict__ out_v, float* __restrict__ q_out, int n_chunks, int n_items, int32_t* __restrict__ tickets,       \
+      float* __restrict__ part_ws
+#define MESSAGE_TC_FWD_ARGS                                                                                                \
+  phi, v_send, v_recv, bptr, ngroups, rec, Wf, bf, n_recv, F, R, res_s, res_v, v_is_zero, out_s, out_v, q_out, n_chunks,    \
+      n_items, tickets, part_ws
+
+template <int KS, int RC, int NSUB, bool ONE>
+__device__ __forceinline__ void message_tc_fwd_body(MESSAGE_TC_FWD_PARAMS) {
   CGVAE_KERNEL_PROLOGUE();
   constexpr int GB = NB / RC;                  // groups per batch
   constexpr int GPW = GB / NSUB;               // groups per consumer warp and batch
@@ -406,7 +417,7 @@ __global__ void __launch_bounds__((4 * NSUB + 2) * 32, 1) message_tc_fwd_kernel(
         bar_wait(sbase + M::D_EMPTY + 8 * buf, ((bc / NDBUF) & 1u) ^ 1u);
         tc_fence_after();
         if (elect_one()) {
-          issue_filter_mmas<KS>(sbase + M::STAGES + s * REC_BYTES, tmem_base, Cols<KS>::D + buf * (KS * NB));
+          issue_filter_mmas<KS, ONE>(sbase + M::STAGES + s * REC_BYTES, tmem_base, Cols<KS>::D + buf * (KS * NB));
           umma_commit_a(sbase + M::D_FULL + 8 * buf);
         }
         __syncwarp();
@@ -668,6 +679,18 @@ __global__ void __launch_bounds__((4 * NSUB + 2) * 32, 1) message_tc_fwd_kernel(
   }
 }
 
+// 3xTF32 filter (default) and 1xTF32 filter (cgvae_set_matmul_precision(1)): same records, same work partition
+template <int KS, int RC, int NSUB>
+__global__ void __launch_bounds__((4 * NSUB + 2) * 32, 1) message_tc_fwd_kernel(MESSAGE_TC_FWD_PARAMS) {
+  message_tc_fwd_body<KS, RC, NSUB, false>(MESSAGE_TC_FWD_ARGS);
+}
+template <int KS, int RC, int NSUB>
+__global__ void __launch_bounds__((4 * NSUB + 2) * 32, 1) message_tc1_fwd_kernel(MESSAGE_TC_FWD_PARAMS) {
+  message_tc_fwd_body<KS, RC, NSUB, true>(MESSAGE_TC_FWD_ARGS);
+}
+#undef MESSAGE_TC_FWD_PARAMS
+#undef MESSAGE_TC_FWD_ARGS
+
 }  // namespace mtc
 }  // namespace cgvae
 
@@ -746,15 +769,18 @@ int cgvae_message_tc_fwd(int n_split, const float* phi, const float* v_send, con
   const size_t tick_bytes = ((size_t)n_items * 4 + 255) / 256 * 256;
   float* part_ws = reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + tick_bytes);
   CGVAE_ZERO(tickets, tick_bytes, st);
+  // the precision mode picks the kernel only (cgvae_set_matmul_precision): records, grid and partition are the same
+  const int one = matmul_precision() == 1 ? 1 : 0;
 #define LAUNCH_TC_FWD(KS, RCV, NSUB)                                                                                             \
   do {                                                                                                                           \
-    static bool attr_done = false;                                                                                               \
+    static bool attr_done[2] = {false, false};                                                                                   \
     constexpr size_t smb = mtc::Map<NSUB, RCV*(KS == 4 ? 7 : 4)>::BYTES;                                                   \
-    if (!attr_done) {                                                                                                            \
-      CGVAE_CUDA(cudaFuncSetAttribute(mtc::message_tc_fwd_kernel<KS, RCV, NSUB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smb)); \
-      attr_done = true;                                                                                                          \
+    auto kernel = one ? mtc::message_tc1_fwd_kernel<KS, RCV, NSUB> : mtc::message_tc_fwd_kernel<KS, RCV, NSUB>;               \
+    if (!attr_done[one]) {                                                                                                       \
+      CGVAE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smb));                            \
+      attr_done[one] = true;                                                                                                     \
     }                                                                                                                            \
-    launch_kernel(mtc::message_tc_fwd_kernel<KS, RCV, NSUB>, grid, dim3((4 * NSUB + 2) * 32), smb, st, phi, v_send, v_recv, bptr, ngroups, \
+    launch_kernel(kernel, grid, dim3((4 * NSUB + 2) * 32), smb, st, phi, v_send, v_recv, bptr, ngroups,                          \
                   recp, Wf, bf, n_recv, F, R, res_s, res_v, v_is_zero, out_s, out_v, q, (int)n_chunks, (int)n_items, tickets,    \
                   part_ws);                                                                                                      \
   } while (0)

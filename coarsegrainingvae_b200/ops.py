@@ -4,6 +4,8 @@ Every function here takes CUDA tensors, allocates outputs / scratch with torch (
 memory), and launches hand-written sm_100a kernels on the current stream through ctypes.  There is no
 CPU path: a non-CUDA tensor raises.  Layouts: scalars [N,F]; vectors planar [N,3,F]; phi [N,K,F].
 """
+import contextlib as _contextlib
+
 import numpy as np
 import torch
 
@@ -1017,6 +1019,40 @@ def adam_clip_step(p, g, m, v, step, max_norm, lr, betas=(0.9, 0.999), eps=1e-8,
 def set_pdl(on):
     """programmatic dependent launch on / off for subsequent launches; returns the previous setting."""
     return bool(_lib.load().cgvae_set_pdl(int(bool(on))))
+
+
+MATMUL_PRECISIONS = ("highest", "high")
+
+
+def set_matmul_precision(mode):
+    """precision of the tensor-core contractions for every launch from now on; returns the previous mode.
+
+    "highest" (the default): 3xTF32, fp32 parity.  "high": 1xTF32, operands rounded to nearest TF32 with fp32
+    accumulation, within 4 * 2^-11 scale-relative per contraction.  It covers the tcgen05 GEMMs (>= 64 rows) and the
+    filter of the tensor-core message forward; every other kernel stays fp32 in both modes.  Independent of
+    torch.get_float32_matmul_precision().  CUDA graphs replay the kernels they were captured with."""
+    if mode not in MATMUL_PRECISIONS:
+        raise ValueError("matmul precision must be one of %s, got %r" % (MATMUL_PRECISIONS, mode))
+    rc = _lib.load().cgvae_set_matmul_precision(MATMUL_PRECISIONS.index(mode))
+    if rc < 0:
+        _lib.check(rc, "set_matmul_precision")
+    return MATMUL_PRECISIONS[rc]
+
+
+def get_matmul_precision():
+    """the current mode of set_matmul_precision: "highest" or "high"."""
+    return MATMUL_PRECISIONS[_lib.load().cgvae_get_matmul_precision()]
+
+
+@_contextlib.contextmanager
+def matmul_precision(mode):
+    """``with matmul_precision("high"): ...`` -- the mode inside the block, the previous one restored on exit (also on an
+    exception)."""
+    prev = set_matmul_precision(mode)
+    try:
+        yield
+    finally:
+        set_matmul_precision(prev)
 
 
 def register_const_range(t):

@@ -661,6 +661,8 @@ class GraphedTrainStep(object):
         import torch.distributed as dist
         self.distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size(trainer.group) > 1
         before = ops.launch_count()
+        # the precision mode the kernels were captured with: a replay runs those kernels whatever the mode is later
+        self.matmul_precision = ops.get_matmul_precision()
         self.graph = torch.cuda.CUDAGraph()
         self.opt_graph = None
         if not self.distributed or trainer.n_overlap:
@@ -812,6 +814,7 @@ class GraphedSampler(object):
             for _ in range(2):
                 self._run()
         torch.cuda.synchronize()
+        self.matmul_precision = ops.get_matmul_precision()      # replays keep the kernels of this mode
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph, stream=side):
             self.out = self._run()
@@ -856,6 +859,7 @@ class ShardedGraphedSampler(object):
         self.per = (self.n_ensemble + self.world - 1) // self.world
         self.mine = [m for m in range(self.n_ensemble) if m % self.world == self.rank]
         self.local = GraphedSampler(model, example_batch, self.per)
+        self.matmul_precision = self.local.matmul_precision
         dev = self.local.eps.device
         self._eps_local = torch.zeros_like(self.local.eps)
         self._mine_idx = torch.tensor(self.mine, dtype=torch.int64, device=dev)

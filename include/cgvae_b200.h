@@ -368,6 +368,17 @@ int cgvae_sample_quality(const float* ref_xyz, const float* samples, const float
 /* Programmatic dependent launch for every launch of the library from now on (default on; CGVAE_PDL=0); returns the previous
  * setting.  Launches already captured in a CUDA graph keep the edges they were captured with. */
 int cgvae_set_pdl(int on);
+/* Precision of the tensor-core contractions for every launch from now on; returns the previous mode.
+ *   0 = 3xTF32, fp32 parity (1e-5 relative); the default, like torch.set_float32_matmul_precision("highest");
+ *   1 = 1xTF32, operands rounded to nearest TF32 (10-bit mantissa), fp32 accumulation, like torch's "high": stated bound
+ *       4 * 2^-11 scale-relative per contraction with zero-mean operands.
+ * It covers the tcgen05 GEMMs (>= 64 rows) and the filter of cgvae_message_tc_fwd; everything else stays fp32 in both
+ * modes (SIMT GEMM tiles, weight-streaming GEMMs, cgvae_wgrad_grouped, cgvae_colsum, the message backward, the 9-split
+ * kernels).  The dispatch (tiles, split-K, grid) is the same in both modes.  Launches already captured in a CUDA graph keep
+ * the kernels they were captured with.  Any other mode: argument error, mode unchanged. */
+int cgvae_set_matmul_precision(int mode);
+/* the current mode of cgvae_set_matmul_precision (0 or 1) */
+int cgvae_get_matmul_precision(void);
 /* Declare [p, p + bytes) a parameter range: memory no kernel writes between two optimiser steps (the flat parameter buffer of
  * a training step).  With programmatic dependent launch enabled (CGVAE_PDL, default on) the weight-streaming GEMMs fetch a
  * weight matrix inside such a range BEFORE their dependency wait, overlapping the copy with the preceding kernel.  Ranges that
