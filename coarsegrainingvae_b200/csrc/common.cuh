@@ -65,8 +65,8 @@ inline int launched(const char* what) {
 // not the work, dominates.  Every kernel of this library starts with pdl_wait() (griddepcontrol.wait: blocks until the
 // preceding grid has completed and flushed its writes -- all global-memory accesses come after it, so ordering is exactly
 // that of a plain stream) and pdl_trigger() (griddepcontrol.launch_dependents: lets the NEXT kernel's launch and prologue
-// overlap with this kernel's execution).  Launches carry cudaLaunchAttributeProgrammaticStreamSerialization when
-// CGVAE_PDL=1 (opt-in: it did not pay on B200 for this workload, see graph.cu::pdl_enabled).
+// overlap with this kernel's execution).  Launches carry cudaLaunchAttributeProgrammaticStreamSerialization while
+// pdl_enabled() (on by default; CGVAE_PDL=0 or cgvae_set_pdl(0) turn it off, see graph.cu).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 #define CGVAE_KERNEL_PROLOGUE() \
@@ -81,19 +81,45 @@ int matmul_precision();
 // inside a parameter range registered with cgvae_register_const_range, and PDL on (gemm_stream.cu)
 bool weights_are_constant(const void* p, size_t bytes);
 
+// cluster == nullptr: no cluster attribute.  The PDL attribute is attached while pdl_enabled().
 template <typename... KArgs, typename... Args>
-inline void launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+inline void launch_with_attrs(void (*kernel)(KArgs...), dim3 grid, dim3 block, const dim3* cluster, size_t smem, cudaStream_t st,
+                              Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[2];
+  unsigned n = 0;
+  if (cluster != nullptr) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = cluster->x;
+    attr[n].val.clusterDim.y = cluster->y;
+    attr[n].val.clusterDim.z = cluster->z;
+    ++n;
+  }
+  if (pdl_enabled()) {
+    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = n;
   (void)cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // errors surface through launched()
+}
+
+template <typename... KArgs, typename... Args>
+inline void launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
+  launch_with_attrs(kernel, grid, block, nullptr, smem, st, args...);
+}
+
+// thread-block cluster of shape `cluster` (every grid extent a multiple of it); a cluster of one CTA is still a cluster
+// launch: the kernels that call cooperative_groups::this_cluster() need the attribute whatever its size
+template <typename... KArgs, typename... Args>
+inline void launch_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, dim3 cluster, size_t smem, cudaStream_t st,
+                           Args... args) {
+  launch_with_attrs(kernel, grid, block, &cluster, smem, st, args...);
 }
 
 // Zero fill as a KERNEL.  Inside a captured CUDA graph a memset node costs 3..11 us of idle time before the next kernel

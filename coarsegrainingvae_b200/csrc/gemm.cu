@@ -116,8 +116,7 @@ struct TileLoader {
 template <int BM, int BN, int BK, int TM, int TN, bool A_KC, bool B_KC, bool CLUSTER>
 __global__ void __launch_bounds__((BM / TM) * (BN / TN)) gemm_kernel(
     const float* __restrict__ A, int64_t lda, const float* __restrict__ B, int64_t ldb, float* __restrict__ C, int64_t ldc,
-    int64_t M, int64_t N, int64_t K, int64_t k_per_split, Epilogue ep, float* __restrict__ partial,
-    int* __restrict__ counters, bool a_vec, bool b_vec) {
+    int64_t M, int64_t N, int64_t K, int64_t k_per_split, Epilogue ep, float* __restrict__ partial, bool a_vec, bool b_vec) {
   CGVAE_KERNEL_PROLOGUE();
   constexpr int NT = (BM / TM) * (BN / TN);
   using LoaderA = TileLoader<BM, BK, A_KC, NT>;
@@ -250,27 +249,6 @@ __global__ void __launch_bounds__((BM / TM) * (BN / TN)) gemm_kernel(
         if (nb + j < N) dst[m * ldd + nb + j] = o[j];
     }
   }
-  if (!split || counters == nullptr) return;
-  // Deterministic split-K without a second launch: every CTA of an output tile publishes its partial sums, the LAST
-  // one to arrive (ticket counter) adds all slices in slice order 0..S-1 -- a fixed order, independent of which CTA
-  // happens to be last -- applies the epilogue and re-arms the counter for the next launch.
-  __shared__ int ticket_sh;
-  __threadfence();
-  __syncthreads();
-  const int tile_id = blockIdx.y * gridDim.x + blockIdx.x;
-  if (tid == 0) ticket_sh = atomicAdd(&counters[tile_id], 1);
-  __syncthreads();
-  if (ticket_sh != (int)gridDim.z - 1) return;
-  __threadfence();
-  const int splits = gridDim.z;
-  for (int idx = tid; idx < BM * BN; idx += NT) {
-    const int64_t m = m0 + idx / BN, n = n0 + idx % BN;
-    if (m >= M || n >= N) continue;
-    float v = 0.f;
-    for (int z = 0; z < splits; ++z) v += __ldcg(partial + ((int64_t)z * M + m) * N + n);
-    C[m * ldc + n] = apply_epilogue(ep, v, m, n, ldc);
-  }
-  if (tid == 0) counters[tile_id] = 0;
 }
 
 __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restrict__ partial, int splits, int64_t M, int64_t N,
@@ -491,255 +469,14 @@ __global__ void __launch_bounds__(1024) colsum_tall_kernel(const float* __restri
   cluster.sync();
 }
 
-// ------------------------------------------------------------------------------------------------------------
-// 3xTF32 warp-MMA kernel for mid-size problems (64 <= M: the 350-row atom-level layers of chignolin, the weight
-// gradients of the protein configs).  The 64x64 SIMT tile above is bound by shared-memory loads (2 LDS.128 per 16 FMA:
-// 13..20 TFLOP/s at these sizes); here a warp owns a 32x32 sub-tile as 2x4 mma.sync.m16n8k8 fragments, the fp32
-// operands are split in registers (hi = tf32(x), lo = tf32(x - hi)) and every product is lo*hi + hi*lo + hi*hi with fp32
-// accumulation: fp32-class accuracy (validated against float64 like the other paths) at the rate of the tensor pipe
-// (measured on this B200, tools/hmma_bench.cu: one m16n8k8 per 2.15 SM-cycles = 92 TFLOP/s fp32-equivalent after the
-// factor 3).  Operand staging, register prefetch, split-K (cluster DSMEM / workspace) and epilogue are those of
-// gemm_kernel; the k-major tiles use a row stride = 8 (mod 32) so that the scalar fragment loads are conflict-free.
-// ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t tf32_hi(float x) {
-  uint32_t r;
-  asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-  return r;
-}
-__device__ __forceinline__ void tf32_split(float x, uint32_t& hi, uint32_t& lo) {
-  hi = tf32_hi(x);
-  lo = tf32_hi(x - __uint_as_float(hi));
-}
-__device__ __forceinline__ void mma_tf32(float (&d)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-
-constexpr int MMA_BM = 64, MMA_BN = 64, MMA_BK = 16, MMA_NT = 128, MMA_PAD = 8;
-
-template <bool A_KC, bool B_KC, bool CLUSTER>
-__global__ void __launch_bounds__(MMA_NT) gemm_mma_kernel(
-    const float* __restrict__ A, int64_t lda, const float* __restrict__ B, int64_t ldb, float* __restrict__ C, int64_t ldc,
-    int64_t M, int64_t N, int64_t K, int64_t k_per_split, Epilogue ep, float* __restrict__ partial, bool a_vec, bool b_vec) {
-  CGVAE_KERNEL_PROLOGUE();
-  constexpr int BM = MMA_BM, BN = MMA_BN, BK = MMA_BK, NT = MMA_NT;
-  using LoaderA = TileLoader<BM, BK, A_KC, NT, MMA_PAD>;
-  using LoaderB = TileLoader<BN, BK, B_KC, NT, MMA_PAD>;
-  static_assert(!LoaderA::ROWMAJOR && !LoaderB::ROWMAJOR, "k-major tiles expected");
-  constexpr int SA = LoaderA::SMEM_FLOATS, SB = LoaderB::SMEM_FLOATS;
-  constexpr int LDA_S = BM + MMA_PAD, LDB_S = BN + MMA_PAD;
-  constexpr int TILE_FLOATS = 2 * (SA + SB);
-  constexpr int SMEM_FLOATS = (CLUSTER && BM * BN > TILE_FLOATS) ? BM * BN : TILE_FLOATS;
-  __shared__ __align__(16) float smem_all[SMEM_FLOATS];
-  float (*As)[SA] = reinterpret_cast<float (*)[SA]>(smem_all);
-  float (*Bs)[SB] = reinterpret_cast<float (*)[SB]>(smem_all + 2 * SA);
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  const int wm = (warp >> 1) * 32, wn = (warp & 1) * 32;
-  const int64_t m0 = (int64_t)blockIdx.y * BM, n0 = (int64_t)blockIdx.x * BN;
-  const int64_t kbeg = (int64_t)blockIdx.z * k_per_split;
-  const int64_t kend = min(K, kbeg + k_per_split);
-
-  constexpr int kFold = 64 / BK;       // fold into `tot` with ordinary (round-to-nearest) fp32 adds every 64 k: the tensor
-                                       // pipe's own accumulation is not round-to-nearest
-  float acc[2][4][4], tot[2][4][4];
-#pragma unroll
-  for (int i = 0; i < 2; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) { acc[i][j][c] = 0.f; tot[i][j][c] = 0.f; }
-
-  constexpr int PD = 2;
-  LoaderA las[PD];
-  LoaderB lbs[PD];
-#pragma unroll
-  for (int p = 0; p < PD; ++p) {
-    if (kbeg + (int64_t)p * BK < kend) {
-      las[p].fetch(A, lda, m0, M, kbeg + (int64_t)p * BK, kend, a_vec, tid);
-      lbs[p].fetch(B, ldb, n0, N, kbeg + (int64_t)p * BK, kend, b_vec, tid);
-    }
-  }
-  int buf = 0, fold = 0;
-  for (int64_t base = kbeg; base < kend; base += (int64_t)PD * BK) {
-#pragma unroll
-    for (int p = 0; p < PD; ++p) {
-      const int64_t k0 = base + (int64_t)p * BK;
-      if (k0 < kend) {
-        las[p].store(As[buf], tid);
-        lbs[p].store(Bs[buf], tid);
-        __syncthreads();
-        if (k0 + (int64_t)PD * BK < kend) {
-          las[p].fetch(A, lda, m0, M, k0 + (int64_t)PD * BK, kend, a_vec, tid);
-          lbs[p].fetch(B, ldb, n0, N, k0 + (int64_t)PD * BK, kend, b_vec, tid);
-        }
-        const float* as = As[buf];
-        const float* bs = Bs[buf];
-#pragma unroll
-        for (int ks = 0; ks < BK / 8; ++ks) {
-          uint32_t ah[2][4], al[2][4], bh[4][2], bl[4][2];
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt) {
-            const float* pa = as + (ks * 8 + t) * LDA_S + wm + mt * 16 + g;
-            tf32_split(pa[0], ah[mt][0], al[mt][0]);
-            tf32_split(pa[8], ah[mt][1], al[mt][1]);
-            tf32_split(pa[4 * LDA_S], ah[mt][2], al[mt][2]);
-            tf32_split(pa[4 * LDA_S + 8], ah[mt][3], al[mt][3]);
-          }
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            const float* pb = bs + (ks * 8 + t) * LDB_S + wn + nt * 8 + g;
-            tf32_split(pb[0], bh[nt][0], bl[nt][0]);
-            tf32_split(pb[4 * LDB_S], bh[nt][1], bl[nt][1]);
-          }
-          // product-major order: eight independent accumulators between two MMAs on the same one (back-to-back MMAs on
-          // one accumulator serialise on the tensor-pipe latency)
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-            for (int nt = 0; nt < 4; ++nt) mma_tf32(acc[mt][nt], al[mt], bh[nt]);
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-            for (int nt = 0; nt < 4; ++nt) mma_tf32(acc[mt][nt], ah[mt], bl[nt]);
-#pragma unroll
-          for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-            for (int nt = 0; nt < 4; ++nt) mma_tf32(acc[mt][nt], ah[mt], bh[nt]);
-        }
-        if (++fold == kFold) {
-          fold = 0;
-#pragma unroll
-          for (int i = 0; i < 2; ++i)
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-#pragma unroll
-              for (int c = 0; c < 4; ++c) { tot[i][j][c] += acc[i][j][c]; acc[i][j][c] = 0.f; }
-        }
-        buf ^= 1;
-      }
-    }
-  }
-#pragma unroll
-  for (int i = 0; i < 2; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) acc[i][j][c] += tot[i][j][c];
-
-  // accumulator fragment: c0,c1 = (row g, cols 2t, 2t+1), c2,c3 = (row g+8, same columns)
-  if constexpr (CLUSTER) {
-    namespace cg = cooperative_groups;
-    cg::cluster_group cluster = cg::this_cluster();
-    __syncthreads();                 // every warp is done reading the operand tiles
-    float* red = smem_all;
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int r = wm + mt * 16 + g + 8 * h, c = wn + nt * 8 + 2 * t;
-          *reinterpret_cast<float2*>(&red[r * BN + c]) = make_float2(acc[mt][nt][2 * h], acc[mt][nt][2 * h + 1]);
-        }
-    cluster.sync();
-    const int S = (int)cluster.num_blocks();
-    const int rank = (int)cluster.block_rank();
-    for (int idx = rank * NT + tid; idx < BM * BN; idx += S * NT) {
-      const int64_t m = m0 + idx / BN, n = n0 + idx % BN;
-      float v = 0.f;
-      for (int z = 0; z < S; ++z) v += *cluster.map_shared_rank(&red[idx], z);
-      if (m < M && n < N) C[m * ldc + n] = apply_epilogue(ep, v, m, n, ldc);
-    }
-    cluster.sync();
-    return;
-  }
-  const bool split = gridDim.z > 1;
-  float* dst = split ? partial + (int64_t)blockIdx.z * M * N : C;
-  const int64_t ldd = split ? N : ldc;
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int64_t m = m0 + wm + mt * 16 + g + 8 * h, n = n0 + wn + nt * 8 + 2 * t;
-        if (m >= M) continue;
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-          if (n + c < N) {
-            const float v = acc[mt][nt][2 * h + c];
-            dst[m * ldd + n + c] = split ? v : apply_epilogue(ep, v, m, n + c, ldc);
-          }
-        }
-      }
-}
-
-static int launch_gemm_mma(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                           int64_t N, int64_t K, const Epilogue& ep, float* ws, size_t ws_bytes, cudaStream_t st) {
-  constexpr int BM = MMA_BM, BN = MMA_BN, BK = MMA_BK;
-  const int64_t tiles = ceil_div(M, BM) * ceil_div(N, BN);
-  const bool a_kc = (form != CGVAE_GEMM_TN), b_kc = (form == CGVAE_GEMM_NT);
-  const bool a_vec = aligned16(A) && (lda % 4 == 0), b_vec = aligned16(B) && (ldb % 4 == 0);
-  // split-K when the output grid leaves SMs idle: cluster (DSMEM reduction) up to 8 slices, else workspace + reduce kernel
-  int S = 1;
-  if (tiles < 2 * kNumSM && K >= 8 * BK) S = (int)std::min<int64_t>(std::min<int64_t>(8, ceil_div(3 * kNumSM, tiles)), ceil_div(K, 128));
-  int64_t kps = ceil_div(ceil_div(K, S), BK) * BK;
-  S = (int)ceil_div(K, kps);
-  if (S > 1 && form != CGVAE_GEMM_TN) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)ceil_div(N, BN), (unsigned)ceil_div(M, BM), (unsigned)S);
-    cfg.blockDim = dim3(MMA_NT);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = (unsigned)S;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    float* nopartial = nullptr;
-    if (b_kc)
-      (void)cudaLaunchKernelEx(&cfg, gemm_mma_kernel<true, true, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, nopartial, a_vec, b_vec);
-    else
-      (void)cudaLaunchKernelEx(&cfg, gemm_mma_kernel<true, false, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, nopartial, a_vec, b_vec);
-    return launched("gemm_mma_cluster");
-  }
-  if (S > 1) {          // TN: deep contraction over the node dimension (weight gradients): workspace split-K
-    const int64_t cap = ws ? (int64_t)(ws_bytes / (sizeof(float) * (size_t)(M * N))) : 1;
-    int want = (int)std::min<int64_t>(ceil_div(3 * kNumSM, tiles), ceil_div(K, 128));
-    S = (int)std::max<int64_t>(1, std::min<int64_t>(want, cap));
-    kps = ceil_div(ceil_div(K, S), BK) * BK;
-    S = (int)ceil_div(K, kps);
-  }
-  dim3 grid((unsigned)ceil_div(N, BN), (unsigned)ceil_div(M, BM), (unsigned)S);
-  float* partial = S > 1 ? ws : nullptr;
-  if (a_kc && b_kc)
-    launch_kernel(gemm_mma_kernel<true, true, false>, dim3(grid), dim3(MMA_NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, partial, a_vec, b_vec);
-  else if (a_kc)
-    launch_kernel(gemm_mma_kernel<true, false, false>, dim3(grid), dim3(MMA_NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, partial, a_vec, b_vec);
-  else
-    launch_kernel(gemm_mma_kernel<false, false, false>, dim3(grid), dim3(MMA_NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, partial, a_vec, b_vec);
-  if (int rc = launched("gemm_mma")) return rc;
-  if (S > 1) {
-    launch_kernel(splitk_reduce_kernel, dim3((unsigned)ceil_div(M * N, 256)), dim3(256), 0, st, (const float*)partial, S, M, N, C, ldc, ep);
-    return launched("gemm_splitk_reduce");
-  }
-  return 0;
-}
-
 template <int BM, int BN, int BK, int TM, int TN>
 static int launch_gemm(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t M,
-                       int64_t N, int64_t K, const Epilogue& ep, float* ws, size_t ws_bytes, int* counters, int n_counters,
-                       cudaStream_t st) {
+                       int64_t N, int64_t K, const Epilogue& ep, float* ws, size_t ws_bytes, cudaStream_t st) {
   constexpr int NT = (BM / TM) * (BN / TN);
   const int64_t tiles = ceil_div(M, BM) * ceil_div(N, BN);
   // split-K only when the output grid leaves most of the 148 SMs idle and K is deep
   int splits = 1;
-  if (ws != nullptr && counters != nullptr && tiles <= n_counters && tiles < kNumSM && K >= 8 * BK) {
+  if (ws != nullptr && tiles < kNumSM && K >= 8 * BK) {
     splits = (int)std::min<int64_t>(ceil_div(2 * kNumSM, tiles), ceil_div(K, 128));
     const int64_t cap = (int64_t)(ws_bytes / (sizeof(float) * (size_t)(M * N)));
     splits = (int)std::max<int64_t>(1, std::min<int64_t>(splits, cap));
@@ -749,51 +486,34 @@ static int launch_gemm(int form, const float* A, int64_t lda, const float* B, in
   if (splits < 1) splits = 1;
   const bool a_kc = (form != CGVAE_GEMM_TN), b_kc = (form == CGVAE_GEMM_NT);
   const bool a_vec = aligned16(A) && (lda % 4 == 0), b_vec = aligned16(B) && (ldb % 4 == 0);
-  static const bool use_cluster = [] { const char* e = getenv("CGVAE_CLUSTER_SPLITK"); return !(e && e[0] == '0'); }();
-  if (use_cluster && tiles < kNumSM && K >= 8 * BK && form != CGVAE_GEMM_TN) {
+  if (tiles < kNumSM && K >= 8 * BK && form != CGVAE_GEMM_TN) {
     // cluster split-K: up to 8 K-slices per output tile (portable cluster size), reduced through DSMEM
     int S = (int)std::min<int64_t>(std::min<int64_t>(8, ceil_div(2 * kNumSM, tiles)), ceil_div(K, 128));
     int64_t kps = ceil_div(ceil_div(K, S), BK) * BK;
     S = (int)ceil_div(K, kps);
     if (S > 1) {
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3((unsigned)ceil_div(N, BN), (unsigned)ceil_div(M, BM), (unsigned)S);
-      cfg.blockDim = dim3(NT);
-      cfg.stream = st;
-      cudaLaunchAttribute attr[2];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 1;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = (unsigned)S;
-      attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      attr[1].val.programmaticStreamSerializationAllowed = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = pdl_enabled() ? 2 : 1;
-      float* nopartial = nullptr;
-      int* nocounters = nullptr;
+      const dim3 grid((unsigned)ceil_div(N, BN), (unsigned)ceil_div(M, BM), (unsigned)S), cluster(1, 1, (unsigned)S);
       if (b_kc)
-        (void)cudaLaunchKernelEx(&cfg, gemm_kernel<BM, BN, BK, TM, TN, true, true, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep,
-                                 nopartial, nocounters, a_vec, b_vec);
+        launch_cluster(gemm_kernel<BM, BN, BK, TM, TN, true, true, true>, grid, dim3(NT), cluster, 0, st, A, lda, B, ldb, C, ldc, M,
+                       N, K, kps, ep, nullptr, a_vec, b_vec);
       else
-        (void)cudaLaunchKernelEx(&cfg, gemm_kernel<BM, BN, BK, TM, TN, true, false, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep,
-                                 nopartial, nocounters, a_vec, b_vec);
+        launch_cluster(gemm_kernel<BM, BN, BK, TM, TN, true, false, true>, grid, dim3(NT), cluster, 0, st, A, lda, B, ldb, C, ldc, M,
+                       N, K, kps, ep, nullptr, a_vec, b_vec);
       return launched("gemm_cluster");
     }
   }
   dim3 grid((unsigned)ceil_div(N, BN), (unsigned)ceil_div(M, BM), (unsigned)splits);
+  // partial sums are added by a second launch: inside a CUDA graph that costs less than an in-kernel "last CTA" fix-up
+  // (fence + ticket: 6.0 vs 5.4 ms per chignolin step on B200)
   float* partial = splits > 1 ? ws : nullptr;
-  // measured on B200 (chignolin step): the in-kernel fix-up (fence + ticket + last-CTA reduction) costs more than the extra
-  // reduce launch inside a CUDA graph (6.0 vs 5.4 ms per step), so it is opt-in
-  static const bool fixup = [] { const char* e = getenv("CGVAE_SPLITK_FIXUP"); return e && e[0] == '1'; }();
-  int* kernel_counters = fixup ? counters : nullptr;   // nullptr: partial sums are reduced by splitk_reduce_kernel
   if (a_kc && b_kc)
-    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, true, true, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, kernel_counters, a_vec, b_vec);
+    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, true, true, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, a_vec, b_vec);
   else if (a_kc && !b_kc)
-    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, true, false, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, kernel_counters, a_vec, b_vec);
+    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, true, false, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, a_vec, b_vec);
   else
-    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, false, false, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, kernel_counters, a_vec, b_vec);
+    launch_kernel(gemm_kernel<BM, BN, BK, TM, TN, false, false, false>, dim3(grid), dim3(NT), 0, st, A, lda, B, ldb, C, ldc, M, N, K, k_per_split, ep, partial, a_vec, b_vec);
   if (int rc = launched("gemm")) return rc;
-  if (splits > 1 && kernel_counters == nullptr) {
+  if (splits > 1) {
     launch_kernel(splitk_reduce_kernel, dim3((unsigned)ceil_div(M * N, 256)), dim3(256), 0, st, (const float*)partial, splits, M, N,
                   C, ldc, ep);
     return launched("gemm_splitk_reduce");
@@ -838,7 +558,7 @@ int cgvae_dense_pair_fwd(const float* x, int64_t ldx, const float* W, int64_t ld
 
 int cgvae_gemm(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t M, int64_t N,
                int64_t K, const float* bias, int act, float* z_out, const float* z_in, int dact, const float* add,
-               void* ws, size_t ws_bytes, int32_t* counters, int n_counters, cgvae_stream_t stream) {
+               void* ws, size_t ws_bytes, int32_t* /*counters*/, int /*n_counters*/, cgvae_stream_t stream) {
   CGVAE_REQUIRE(form >= 0 && form <= 2, "gemm: bad form %d", form);
   CGVAE_REQUIRE(M >= 0 && N >= 0 && K >= 0, "gemm: negative size");
   if (M == 0 || N == 0) return 0;
@@ -861,11 +581,10 @@ int cgvae_gemm(int form, const float* A, int64_t lda, const float* B, int64_t ld
   if (launch_gemm_stream(form, A, lda, B, ldb, C, ldc, M, N, K, bias, act, z_out, z_in, dact, add, st))
     return launched("gemm_stream");
   float* wsf = reinterpret_cast<float*>(ws);
-  static const bool use_skinny = [] { const char* e = getenv("CGVAE_SKINNY_GEMM"); return !(e && e[0] == '0'); }();
   // measured in isolation inside a CUDA graph (tools/bench_skinny.py, weights rotated through > L2): the column-per-thread
   // kernel wins for wide outputs (W2 forward, 5400 columns: 17.9 vs 23.2 us) and loses where 8 cluster slices of 64-wide
   // tiles leave too few threads in flight (N = 600 outputs: 80 CTAs x 64 threads), so it takes the NT form with N >= 1024
-  if (use_skinny && M <= 16 && form == CGVAE_GEMM_NT && K >= 64 && N >= 1024) {
+  if (M <= 16 && form == CGVAE_GEMM_NT && K >= 64 && N >= 1024) {
     // one output column per thread, K split over a cluster of up to 8 CTAs
     const bool b_kc = (form == CGVAE_GEMM_NT);
     const bool a_vec = aligned16(A) && (lda % 4 == 0), b_vec = aligned16(B) && (ldb % 4 == 0);
@@ -875,49 +594,24 @@ int cgvae_gemm(int form, const float* A, int64_t lda, const float* B, int64_t ld
     int S = (int)std::min<int64_t>(std::min<int64_t>(8, std::max<int64_t>(1, ceil_div(2 * kNumSM, tiles))), ceil_div(K, 2 * SK_BK));
     int64_t kps = ceil_div(ceil_div(K, S), SK_BK) * SK_BK;
     S = (int)ceil_div(K, kps);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)tiles, 1, (unsigned)S);
-    cfg.blockDim = dim3(BNs);
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = (unsigned)S;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    const dim3 grid((unsigned)tiles, 1, (unsigned)S), cluster(1, 1, (unsigned)S);
     if (narrow) {
-      if (b_kc) (void)cudaLaunchKernelEx(&cfg, gemm_skinny_kernel<64, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
-      else (void)cudaLaunchKernelEx(&cfg, gemm_skinny_kernel<64, false>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
+      if (b_kc) launch_cluster(gemm_skinny_kernel<64, true>, grid, dim3(BNs), cluster, 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
+      else launch_cluster(gemm_skinny_kernel<64, false>, grid, dim3(BNs), cluster, 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
     } else {
-      if (b_kc) (void)cudaLaunchKernelEx(&cfg, gemm_skinny_kernel<128, true>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
-      else (void)cudaLaunchKernelEx(&cfg, gemm_skinny_kernel<128, false>, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
+      if (b_kc) launch_cluster(gemm_skinny_kernel<128, true>, grid, dim3(BNs), cluster, 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
+      else launch_cluster(gemm_skinny_kernel<128, false>, grid, dim3(BNs), cluster, 0, st, A, lda, B, ldb, C, ldc, M, N, K, kps, ep, a_vec, b_vec);
     }
     return launched("gemm_skinny");
   }
   // skinny problems (decoder graphs: 12..96 rows) stream the weight matrix: deep k-tiles keep 8-16 KB per CTA in flight
-  if (M <= 16) return launch_gemm<16, 32, 64, 1, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, counters, n_counters, st);
-  if (M <= 32) return launch_gemm<32, 32, 64, 2, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, counters, n_counters, st);
+  if (M <= 16) return launch_gemm<16, 32, 64, 1, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, st);
+  if (M <= 32) return launch_gemm<32, 32, 64, 2, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, st);
   if (M <= 48 && form != CGVAE_GEMM_TN)   // UpdateBlock mixes on 12-bead graphs: 36 rows
-    return launch_gemm<48, 32, 32, 3, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, counters, n_counters, st);
-  // 3xTF32 on the warp-level tensor path (gemm_mma_kernel): opt-in (CGVAE_MMA_GEMM=1).  Measured on B200 at the shapes of
-  // this workload (tools/bench_mid_gemm.py) it is no faster than the SIMT tile (350 x 600 <- 1800: 42 vs 43 us; 2000 x 1536
-  // x 512 weight gradient: 127 vs 142 us) and, as every 3xTF32 scheme, it carries a 2^-21 relative error per PRODUCT, which
-  // one ill-conditioned weight gradient of the PCN parity test turns into 1.08e-5 (gate: 1e-5); fp32 FMA has no
-  // product error.  It stays in the library as the starting point of a TMA-fed multi-stage version.
-  static const bool use_mma = [] { const char* e = getenv("CGVAE_MMA_GEMM"); return e && e[0] == '1'; }();
-  if (use_mma && M >= 64 && N >= 32 && K >= 16 && form != CGVAE_GEMM_TN)
-    return launch_gemm_mma(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, st);
-  // 128-row tiles, 8x4 per thread (3 LDS.128 per 32 FMA instead of 2 per 16; the 64x64 tile is bound by shared-memory
-  // loads: ncu short-scoreboard stalls, 37 % issue utilisation).  Measured on B200 at the chignolin atom-level layers
-  // (350 rows): NN 35 vs 39 us, but NT 22 vs 19.5 and TN 59 vs 52 us (3 row tiles of 128 waste 9 % and halve the CTA
-  // count), 3.55 vs 3.49 ms per step -- opt-in
-  static const bool tall = [] { const char* e = getenv("CGVAE_GEMM_TALL"); return e && e[0] == '1'; }();
-  if (tall && M >= 192 && N >= 64)
-    return launch_gemm<128, 64, 16, 8, 4>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, counters, n_counters, st);
-  return launch_gemm<64, 64, 16, 4, 4>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, counters, n_counters, st);
+    return launch_gemm<48, 32, 32, 3, 2>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, st);
+  // 64x64 tiles: a 128x64 tile with 8x4 per thread measured slower on B200 at the chignolin atom-level layers (350 rows,
+  // 3.55 vs 3.49 ms per step): 3 row tiles of 128 waste 9 % and halve the CTA count
+  return launch_gemm<64, 64, 16, 4, 4>(form, A, lda, B, ldb, C, ldc, M, N, K, ep, wsf, ws_bytes, st);
 }
 
 int cgvae_colsum(const float* X, int64_t ldx, int64_t M, int64_t N, float* out, cgvae_stream_t stream) {
@@ -927,20 +621,8 @@ int cgvae_colsum(const float* X, int64_t ldx, int64_t M, int64_t N, float* out, 
     const int blocks = (int)ceil_div(N, 32);
     int S = (int)std::min<int64_t>(8, std::max<int64_t>(1, (2 * kNumSM) / blocks));
     while (S & (S - 1)) S &= S - 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)blocks, (unsigned)S, 1);
-    cfg.blockDim = dim3(32, 32, 1);
-    cfg.stream = (cudaStream_t)stream;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 1;
-    attr[0].val.clusterDim.y = (unsigned)S;
-    attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = pdl_enabled() ? 2 : 1;
-    (void)cudaLaunchKernelEx(&cfg, colsum_tall_kernel, X, ldx, M, N, out);
+    launch_cluster(colsum_tall_kernel, dim3((unsigned)blocks, (unsigned)S, 1), dim3(32, 32, 1), dim3(1, (unsigned)S, 1), 0,
+                   (cudaStream_t)stream, X, ldx, M, N, out);
     return launched("colsum_tall");
   }
   launch_kernel(colsum_kernel, dim3((unsigned)ceil_div(N, 32)), dim3(dim3(32, 8)), 0, (cudaStream_t)stream, X, ldx, M, N, out);

@@ -437,21 +437,8 @@ static bool launch_nn(const float* G, int64_t ldg, const float* W, int64_t ldw, 
     }
     attr_bytes = kMaxStreamSmem;
   }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)blocks, 1, (unsigned)S);
-  cfg.blockDim = dim3(NW * 32);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 1;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = (unsigned)S;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
-  (void)cudaLaunchKernelEx(&cfg, gemm_nn_stream_kernel<MR, VEC, NW>, map, G, ldg, C, ldc, M, N, K, k_per_cta, box_rows, ep, w_const);
+  launch_cluster(gemm_nn_stream_kernel<MR, VEC, NW>, dim3((unsigned)blocks, 1, (unsigned)S), dim3(NW * 32), dim3(1, 1, (unsigned)S), smem,
+                 st, map, G, ldg, C, ldc, M, N, K, k_per_cta, box_rows, ep, w_const);
   return true;
 }
 
@@ -459,8 +446,7 @@ static bool launch_nn(const float* G, int64_t ldg, const float* W, int64_t ldw, 
 int launch_gemm_stream(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t M,
                        int64_t N, int64_t K, const float* bias, int act, float* z_out, const float* z_in, int dact,
                        const float* add, cudaStream_t st) {
-  static const bool enabled = [] { const char* e = getenv("CGVAE_STREAM_GEMM"); return !(e && e[0] == '0'); }();
-  if (!enabled || M > 48 || M < 1 || form == CGVAE_GEMM_TN) return 0;
+  if (M > 48 || M < 1 || form == CGVAE_GEMM_TN) return 0;
   if (N * K < 64 * 64 || N >= (1 << 24) || K >= (1 << 24)) return 0;
   const StreamEpilogue ep{bias, act, z_out, z_in, dact, add, nullptr, 0, 0};
   const int m = (int)M, n = (int)N, k = (int)K;
@@ -477,19 +463,15 @@ int launch_gemm_stream(int form, const float* A, int64_t lda, const float* B, in
   const bool wide = ceil_div(N, 64) * 2 > kNumSM;       // many columns: 128-column panels keep the grid within one wave
   if (M <= 12) return wide ? launch_nn<12, 4, 16>(A, lda, B, ldb, C, ldc, m, n, k, ep, st) : launch_nn<12, 2, 16>(A, lda, B, ldb, C, ldc, m, n, k, ep, st);
   if (M <= 16) return wide ? launch_nn<16, 4, 16>(A, lda, B, ldb, C, ldc, m, n, k, ep, st) : launch_nn<16, 2, 16>(A, lda, B, ldb, C, ldc, m, n, k, ep, st);
-  // 17..48 rows: measured on B200 (tools/bench_skinny.py, M = 36): the cluster split-K tiles of gemm.cu are as fast or
-  // faster (8.0 vs 9.0 us at 600x600, 10.6 vs 12.4 us at 600x1200) -- the G^T broadcasts dominate the panel math
-  static const bool nn_wide_rows = [] { const char* e = getenv("CGVAE_STREAM_NN_ROWS48"); return e && e[0] == '1'; }();
-  if (!nn_wide_rows) return 0;
-  if (M <= 36) return launch_nn<36, 2, 8>(A, lda, B, ldb, C, ldc, m, n, k, ep, st);
-  return launch_nn<48, 2, 8>(A, lda, B, ldb, C, ldc, m, n, k, ep, st);
+  // 17..48 rows: measured on B200 (tools/bench_skinny.py, M = 36), 36- and 48-row panels were slower than the cluster
+  // split-K tiles of gemm.cu (9.0 vs 8.0 us at 600x600, 12.4 vs 10.6 us at 600x1200): the G^T broadcasts dominate the math
+  return 0;
 }
 
 // two Dense layers on the same input, weights adjacent in memory: W = [W1 (N1 rows); W2 (N2 rows)], no bias / activation
 int launch_dense_pair_stream(const float* X, int64_t ldx, const float* W, int64_t ldw, float* C1, int64_t ldc1, float* C2,
                              int64_t ldc2, int64_t M, int64_t N1, int64_t N2, int64_t K, cudaStream_t st) {
-  static const bool enabled = [] { const char* e = getenv("CGVAE_STREAM_GEMM"); return !(e && e[0] == '0'); }();
-  if (!enabled || M > 48 || M < 1 || N1 + N2 >= (1 << 24) || K >= (1 << 24)) return 0;
+  if (M > 48 || M < 1 || N1 + N2 >= (1 << 24) || K >= (1 << 24)) return 0;
   if (K % 4 != 0 || K < 128 || ldx % 4 != 0 || ldw % 4 != 0 || !aligned16(X) || !aligned16(W)) return 0;
   const StreamEpilogue ep{nullptr, 0, nullptr, nullptr, 0, nullptr, C2, (int)N1, ldc2};
   const int m = (int)M, n = (int)(N1 + N2), k = (int)K;

@@ -50,6 +50,7 @@ constexpr uint32_t TMEM_COLS = 512;
 static_assert((1 + NBIG) * BN <= (int)TMEM_COLS, "accumulators must fit in TMEM");
 constexpr int PS = BN + 4;                                             // row stride (floats) of a parked partial tile
 constexpr int MAX_KT_PER_CTA = 96;   // longest accumulation chain per CTA (k-steps of 32): keeps the 1e-5 gate with margin
+constexpr int MIN_M = 64;            // fewer rows: the SIMT tiles and the weight-streaming kernels (gemm.cu, gemm_stream.cu)
 
 struct Ep {
   const float* bias;
@@ -249,7 +250,7 @@ struct Ring {
 // the split warps' pass over one landed stage: 3xTF32 writes the lo tile next to the raw one; 1xTF32 rounds the raw tile
 // to nearest TF32 in place (the tensor core would truncate: a one-sided error that grows with K instead of averaging out)
 template <bool ONE, int NT>
-__device__ __forceinline__ void split_stage(char* stage, int t, int split_mode) {
+__device__ __forceinline__ void split_stage(char* stage, int t) {
   const float4* raw = reinterpret_cast<const float4*>(stage);
   constexpr int PER = (int)(RAW_BYTES / 16) / NT;   // 8 float4 per thread
   float4 x[PER];
@@ -262,29 +263,14 @@ __device__ __forceinline__ void split_stage(char* stage, int t, int split_mode) 
       rawm[t + it * NT] = make_float4(to_tf32(x[it].x), to_tf32(x[it].y), to_tf32(x[it].z), to_tf32(x[it].w));
   } else {
     float4* lo = reinterpret_cast<float4*>(stage + RAW_BYTES);
-    if (split_mode == 0) {
 #pragma unroll
-      for (int it = 0; it < PER; ++it) {
-        float4 l;
-        l.x = lo_of(x[it].x);
-        l.y = lo_of(x[it].y);
-        l.z = lo_of(x[it].z);
-        l.w = lo_of(x[it].w);
-        lo[t + it * NT] = l;
-      }
-    } else {
-      // round-to-nearest hi written back over the raw tile: |lo| <= 2^-12 |x| keeps one more bit than the truncating split
-      float4* rawm = reinterpret_cast<float4*>(stage);
-#pragma unroll
-      for (int it = 0; it < PER; ++it) {
-        float4 h, l;
-        split_tf32(x[it].x, h.x, l.x);
-        split_tf32(x[it].y, h.y, l.y);
-        split_tf32(x[it].z, h.z, l.z);
-        split_tf32(x[it].w, h.w, l.w);
-        rawm[t + it * NT] = h;
-        lo[t + it * NT] = l;
-      }
+    for (int it = 0; it < PER; ++it) {
+      float4 l;
+      l.x = lo_of(x[it].x);
+      l.y = lo_of(x[it].y);
+      l.z = lo_of(x[it].z);
+      l.w = lo_of(x[it].w);
+      lo[t + it * NT] = l;
     }
   }
 }
@@ -305,8 +291,8 @@ __device__ __forceinline__ void load_acc1(uint32_t taddr, bool any, float (&out)
 
 template <bool A_KC, bool B_KC, bool ONE>
 __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUtensorMap& map_b, float* __restrict__ C, int64_t ldc,
-                                             int64_t M, int64_t N, int64_t K, int kt_per_split, const Ep& ep, int split_mode,
-                                             int cluster_size, float* __restrict__ partial, int b_const) {
+                                             int64_t M, int64_t N, int64_t K, int kt_per_split, const Ep& ep, int cluster_size,
+                                             float* __restrict__ partial, int b_const) {
   constexpr int STAGES = Ring<ONE>::STAGES;
   constexpr uint32_t STAGE_BYTES = Ring<ONE>::STAGE_BYTES;
   // b_const: B is a weight matrix inside a registered parameter range -- the producer issues its first tiles BEFORE the
@@ -376,7 +362,7 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
     for (int i = 0; i < nkt; ++i) {
       const int s = i % STAGES;
       mbar_wait(&raw_full[s], (uint32_t)(i / STAGES) & 1u);
-      split_stage<ONE, NUM_SPLIT_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, tid, split_mode);
+      split_stage<ONE, NUM_SPLIT_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, tid);
       fence_async_smem();            // generic-proxy writes -> visible to the tensor core (async proxy)
       __syncwarp();
       if (lane == 0) mbar_arrive(&lo_done[s]);
@@ -427,7 +413,6 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
             const uint32_t d_big = tmem_base + (uint32_t)(1 + i % NBIG) * BN;
             umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_hi + bo), (i > 0 || ks > 0) ? 1u : 0u, idesc);
             umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
-            if (split_mode == 2) umma_tf32_ss(tmem_base, make_desc_op<A_KC>(a_lo + ao), make_desc_op<B_KC>(b_lo + bo), 1u, idesc);
             umma_tf32_ss(d_big, make_desc_op<A_KC>(a_hi + ao), make_desc_op<B_KC>(b_hi + bo), (i >= NBIG || ks > 0) ? 1u : 0u, idesc);
           }
         }
@@ -505,15 +490,14 @@ __device__ __forceinline__ void gemm_tc_body(const CUtensorMap& map_a, const CUt
 
 #define GEMM_TC_PARAMS                                                                                                          \
   const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b, float* __restrict__ C, int64_t ldc,    \
-      int64_t M, int64_t N, int64_t K, int kt_per_split, Ep ep, int split_mode, int cluster_size, float* __restrict__ partial, \
-      int b_const
+      int64_t M, int64_t N, int64_t K, int kt_per_split, Ep ep, int cluster_size, float* __restrict__ partial, int b_const
 template <bool A_KC, bool B_KC>
 __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc_kernel(GEMM_TC_PARAMS) {
-  gemm_tc_body<A_KC, B_KC, false>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, split_mode, cluster_size, partial, b_const);
+  gemm_tc_body<A_KC, B_KC, false>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, cluster_size, partial, b_const);
 }
 template <bool A_KC, bool B_KC>
 __global__ void __launch_bounds__(NUM_THREADS, 1) gemm_tc1_kernel(GEMM_TC_PARAMS) {
-  gemm_tc_body<A_KC, B_KC, true>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, split_mode, cluster_size, partial, b_const);
+  gemm_tc_body<A_KC, B_KC, true>(map_a, map_b, C, ldc, M, N, K, kt_per_split, ep, cluster_size, partial, b_const);
 }
 #undef GEMM_TC_PARAMS
 
@@ -672,7 +656,7 @@ __device__ __forceinline__ void gemm_tc_persistent_body(const CUtensorMap& map_a
       for (int kt = 0; kt < num_kt; ++kt, ++it) {
         const int s = it % STAGES;
         mbar_wait(&raw_full[s], (uint32_t)(it / STAGES) & 1u);
-        split_stage<ONE, P_LO_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, t0, 0);
+        split_stage<ONE, P_LO_WARPS * 32>(smem + (uint32_t)s * STAGE_BYTES, t0);
         fence_async_smem();
         __syncwarp();
         if (lane == 0) mbar_arrive(&lo_done[s]);
@@ -733,22 +717,11 @@ static bool encode_map(CUtensorMap* map, const float* base, int64_t inner, int64
 
 }  // namespace tc
 
-bool tcgen05_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("CGVAE_TCGEN05");
-    return !(e && e[0] == '0');
-  }();
-  return on;
-}
-
 // returns 1 when the problem was launched on the tensor-core path, 0 when the caller should use the SIMT kernel
 int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc, int64_t M,
                         int64_t N, int64_t K, const float* bias, int act, float* z_out, const float* z_in, int dact,
                         const float* add, float* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!tcgen05_enabled()) return 0;
-  static const int min_m = [] { const char* e = getenv("CGVAE_TC_MIN_M"); return e ? atoi(e) : 64; }();
-  static const int split_mode = [] { const char* e = getenv("CGVAE_TC_SPLIT"); return e ? atoi(e) : 0; }();
-  if (M < min_m || N < 64 || K < 32) return 0;
+  if (M < tc::MIN_M || N < 64 || K < 32) return 0;
   // TMA: 16-byte aligned bases and row pitches
   if (!aligned16(A) || !aligned16(B) || (lda % 4) != 0 || (ldb % 4) != 0) return 0;
   const bool a_kc = (form != CGVAE_GEMM_TN), b_kc = (form == CGVAE_GEMM_NT);
@@ -777,18 +750,8 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
   tc::Ep ep{bias, act, z_out, z_in, dact, add};
   // the precision mode picks the kernel only: S, groups, persistent eligibility and grid are those of the 3xTF32 kernels
   const bool one = matmul_precision() == 1;
-  static const bool persistent_on = [] { const char* e = getenv("CGVAE_TC_PERSISTENT"); return !(e && e[0] == '0'); }();
-  if (persistent_on && S == 1 && groups == 1 && tiles >= 2 * kNumSM && num_kt <= tc::P_MAX_KT) {
-    cudaLaunchConfig_t pc = {};
-    pc.gridDim = dim3((unsigned)std::min<int64_t>(tiles, kNumSM));
-    pc.blockDim = dim3(tc::P_THREADS);
-    pc.dynamicSmemBytes = tc::P_SMEM_BYTES;
-    pc.stream = st;
-    cudaLaunchAttribute pattr[1];
-    pattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    pattr[0].val.programmaticStreamSerializationAllowed = 1;
-    pc.attrs = pattr;
-    pc.numAttrs = pdl_enabled() ? 1 : 0;
+  if (S == 1 && groups == 1 && tiles >= 2 * kNumSM && num_kt <= tc::P_MAX_KT) {
+    const dim3 grid((unsigned)std::min<int64_t>(tiles, kNumSM));
     const int tiles_n = (int)ceil_div(N, tc::BN), n_tiles = (int)tiles;
     static bool p_attr_done[6] = {false, false, false, false, false, false};
     auto pgo = [&](auto kernel, int idx) {
@@ -796,7 +759,7 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
         cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::P_SMEM_BYTES);
         p_attr_done[idx] = true;
       }
-      (void)cudaLaunchKernelEx(&pc, kernel, map_a, map_b, C, ldc, M, N, K, ep, tiles_n, n_tiles);
+      launch_kernel(kernel, grid, dim3(tc::P_THREADS), tc::P_SMEM_BYTES, st, map_a, map_b, C, ldc, M, N, K, ep, tiles_n, n_tiles);
     };
     if (one) {
       if (a_kc && b_kc) pgo(tc::gemm_tc1_persistent_kernel<true, true>, 3);
@@ -811,27 +774,15 @@ int launch_gemm_tcgen05(int form, const float* A, int64_t lda, const float* B, i
   }
   if (groups > 1) ep = tc::Ep{nullptr, 0, nullptr, nullptr, 0, nullptr};
   float* partial = groups > 1 ? ws : nullptr;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)ceil_div(N, tc::BN), (unsigned)ceil_div(M, tc::BM), (unsigned)(S * groups));
-  cfg.blockDim = dim3(tc::NUM_THREADS);
-  cfg.dynamicSmemBytes = tc::SMEM_BYTES;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 1;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = (unsigned)S;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
+  const dim3 grid((unsigned)ceil_div(N, tc::BN), (unsigned)ceil_div(M, tc::BM), (unsigned)(S * groups)), cluster(1, 1, (unsigned)S);
   static bool attr_done[6] = {false, false, false, false, false, false};
   auto go = [&](auto kernel, int idx) {
     if (!attr_done[idx]) {
       cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_BYTES);
       attr_done[idx] = true;
     }
-    (void)cudaLaunchKernelEx(&cfg, kernel, map_a, map_b, C, ldc, M, N, K, kps, ep, split_mode, S, partial, b_const);
+    launch_cluster(kernel, grid, dim3(tc::NUM_THREADS), cluster, tc::SMEM_BYTES, st, map_a, map_b, C, ldc, M, N, K, kps, ep, S, partial,
+                   b_const);
   };
   if (one) {
     if (a_kc && b_kc) go(tc::gemm_tc1_kernel<true, true>, 3);

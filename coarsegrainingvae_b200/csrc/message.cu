@@ -58,7 +58,7 @@ __global__ void __launch_bounds__(kFwdWarps * 32, 5) message_fwd_kernel(
   // A CTA handles recv_per_cta consecutive receivers, kFwdWarps at a time (neighbouring receivers share most of their
   // senders: the gathered 128-byte rows hit L1).  Measured on B200 (c5, 20 000 atoms): one pass of 4 receivers per CTA
   // (dynamic block scheduling, 231 M edges/s) beats 8-warp CTAs (214) and persistent chunks of 64..870 receivers
-  // (193..126): co-resident CTAs of different chunks thrash L1, so recv_per_cta defaults to kFwdWarps.
+  // (193..126): co-resident CTAs of different chunks thrash L1, so the host passes recv_per_cta = kFwdWarps.
   const int64_t i_beg = (int64_t)blockIdx.x * recv_per_cta;
   const int64_t i_end = min(n_recv, i_beg + recv_per_cta);
   // Per-edge metadata (sender index, basis row, unit vector: 68 bytes at RB = 12) is warp-uniform.  Read per edge it was
@@ -628,11 +628,8 @@ int cgvae_message_fwd(int n_split, const float* phi, const float* v_send, const 
   CGVAE_REQUIRE(n_split != 4 || v_is_zero || v_recv, "message_fwd: v_recv missing for the cross block");
   CGVAE_REQUIRE(aligned16(basis) && aligned16(unit), "message_fwd: edge data must be 16-byte aligned");
   const int64_t fy = ceil_div(F, 32);
-  int64_t per = kFwdWarps;
-  static const int forced = [] { const char* e = getenv("CGVAE_FWD_RECV_PER_CTA"); return e ? atoi(e) : 0; }();
-  if (forced > 0) per = ceil_div((int64_t)forced, kFwdWarps) * kFwdWarps;
-  const int recv_per_cta = (int)per;
-  dim3 grid((unsigned)ceil_div(n_recv, per), (unsigned)fy);
+  const int recv_per_cta = kFwdWarps;
+  dim3 grid((unsigned)ceil_div(n_recv, recv_per_cta), (unsigned)fy);
   cudaStream_t st = (cudaStream_t)stream;
 #define LAUNCH_FWD(KS, RBQ)                                                                                            \
   launch_kernel(message_fwd_kernel<KS, RBQ>, dim3(grid), dim3(kFwdWarps * 32), 0, st, phi, v_send, v_recv, rowptr, col, basis, unit, Wf, bf, \

@@ -786,10 +786,9 @@ int cgvae_message_tc_fwd(int n_split, const float* phi, const float* v_send, con
   } while (0)
   if (n_split == 3) {
     // RC = 8 with 8 consumer warps (NSUB = 2: 320 threads, no spills) beats 16 consumer warps at 96 registers (48-byte spill in
-    // the column loop): 76.8 vs 80.7 us at the chignolin atom graph, 15.7 vs 16.2 ms at c5 / 12 A.  CGVAE_MSG_TC_NSUB2=0: old form
-    static const bool nsub2 = [] { const char* e = getenv("CGVAE_MSG_TC_NSUB2"); return !(e && e[0] == '0'); }();
+    // the column loop): 76.8 vs 80.7 us at the chignolin atom graph, 15.7 vs 16.2 ms at c5 / 12 A
     if (RC == 4) LAUNCH_TC_FWD(3, 4, 4);
-    else if (RC == 8) { if (nsub2) LAUNCH_TC_FWD(3, 8, 2); else LAUNCH_TC_FWD(3, 8, 4); }
+    else if (RC == 8) LAUNCH_TC_FWD(3, 8, 2);
     else LAUNCH_TC_FWD(3, 16, 2);
   } else {
     // RC = 8: 56 accumulators per thread only fit with 8 consumer warps (NSUB = 2: 320 threads, 204 registers each)

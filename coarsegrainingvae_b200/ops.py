@@ -410,19 +410,6 @@ def edge_geometry(graph, xyz_send, xyz_recv, n_rbf, cutoff, edge_wgt=None, r_edg
 # --------------------------------------------------------------------------------------------------
 
 _SPLITK_WS_BYTES = 32 << 20
-_N_TICKETS = 1024
-_TICKETS = {}
-
-
-def _tickets(dev, stream):
-    """zero-initialised split-K ticket counters, one array per (device, stream): launches on different streams may run
-    concurrently and must not share tickets; every kernel leaves its tickets at zero."""
-    key = (dev.index, stream)
-    t = _TICKETS.get(key)
-    if t is None:
-        t = torch.zeros(_N_TICKETS, dtype=torch.int32, device=dev)
-        _TICKETS[key] = t
-    return t
 
 
 def gemm(form, A, B, M, N, K, bias=None, act=0, z_out=False, z_in=None, dact=0, add=None, out=None):
@@ -456,14 +443,13 @@ def gemm(form, A, B, M, N, K, bias=None, act=0, z_out=False, z_in=None, dact=0, 
     Z = torch.empty((M, N), dtype=torch.float32, device=dev) if z_out else None
     tiles = ((M + 63) // 64) * ((N + 63) // 64) if M > 32 else ((N + 31) // 32)
     st = _stream()
-    ws = tk = None
+    ws = None
     if (tiles < 148 and K >= 512) or (K > 24576 and M >= 64):      # split-K workspace (SIMT tiles; tcgen05 group partials)
         ws = torch.empty(_SPLITK_WS_BYTES, dtype=torch.uint8, device=dev)
-        tk = _tickets(dev, st)
     t0 = TIMER.begin("gemm") if TIMER is not None else None
     _lib.check(lib.cgvae_gemm(form, _p(A), A.stride(0), _p(B), B.stride(0), _p(C), ldc, M, N, K, _p(bias), act, _p(Z),
-                              _p(z_in), dact, _p(add), _p(ws), _SPLITK_WS_BYTES if ws is not None else 0, _p(tk),
-                              _N_TICKETS if tk is not None else 0, st), "gemm")
+                              _p(z_in), dact, _p(add), _p(ws), _SPLITK_WS_BYTES if ws is not None else 0, None, 0, st),
+               "gemm")
     if t0 is not None:
         meta = dict(form=form, M=M, N=N, K=K, lda=A.stride(0), ldb=B.stride(0))
         if TIMER.keep_operands:

@@ -134,11 +134,10 @@ int cgvae_edge_geometry(const float* xyz_send, const float* xyz_recv, const floa
 /* Dense / nn.Linear forward and backward contractions (modules.py:75-114, conv.py:41-49,568-586).
  * C = epilogue(op(A) op(B)) with epilogue, in order: + bias[N] (nullable); z_out = value (nullable,
  * pre-activation copy, ld = ldc); act; * dact(z_in) when z_in != NULL (activation backward with the
- * saved pre-activation, act code `dact`); + add[M,N] (nullable residual, ld = ldc). fp32 FMA.
- * ws (nullable): scratch for deterministic split-K when the output grid cannot fill 148 SMs; `counters`
- * (nullable with ws): n_counters int32 tickets, ZERO on entry and left zero on exit, not shared between
- * launches that may run concurrently (one array per stream).  The last CTA of each output tile sums the
- * K-slices in slice order, so the result does not depend on scheduling. */
+ * saved pre-activation, act code `dact`); + add[M,N] (nullable residual, ld = ldc).
+ * ws (nullable): ws_bytes of scratch for deterministic split-K when the output grid cannot fill 148 SMs: the
+ * K-slices are written there and a second kernel adds them in slice order, so the result does not depend on
+ * scheduling.  Not shared between launches that may run concurrently.  counters / n_counters are ignored. */
 int cgvae_gemm(int form, const float* A, int64_t lda, const float* B, int64_t ldb, float* C, int64_t ldc,
                int64_t M, int64_t N, int64_t K, const float* bias, int act, float* z_out,
                const float* z_in, int dact, const float* add, void* ws, size_t ws_bytes,

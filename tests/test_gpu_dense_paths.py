@@ -1,9 +1,9 @@
 """GPU (B200): every branch of the dense-contraction dispatcher that the PCN protein step (c4: F = 512, 16 000 beads,
 48 000 planar vector rows) runs, against float64 torch on the device, with the kernel that ran confirmed by the profiler.
 
-The dispatcher is ``cgvae_gemm`` / ``cgvae_colsum`` (csrc/gemm.cu) and ``launch_gemm_tcgen05`` (csrc/gemm_tc.cu).  Paths are
-chosen by shape alone (the CGVAE_* switches are read once per process), so every case names the kernel and grid its shape
-must reach, and ``_probe`` checks them in the CUDA trace:
+The dispatcher is ``cgvae_gemm`` / ``cgvae_colsum`` (csrc/gemm.cu), ``launch_gemm_tcgen05`` (csrc/gemm_tc.cu) and
+``launch_gemm_stream`` (csrc/gemm_stream.cu).  Paths are chosen by shape and alignment alone, so every case names the kernel
+and grid (and for the decoder-sized shapes the block) its shape must reach, and ``_probe`` checks them in the CUDA trace:
 
   * persistent tcgen05 kernel: >= 296 output tiles, K <= 1280, grid.x = 148;
   * one-CTA-per-tile tcgen05 kernel, K split over a cluster of S CTAs (grid.z = S); S = 1 for long K-loops on many tiles;
@@ -11,8 +11,12 @@ must reach, and ``_probe`` checks them in the CUDA trace:
     group partials in order and applies the epilogue;
   * the SIMT gemm_kernel for what TMA cannot take (misaligned bases, ld % 4 != 0) and for group partials that do not
     fit the 32 MB split-K workspace (one unsplit fp32 chain over K);
+  * below 64 rows (decoder graphs: 12 beads, 36 vector rows): the TMA weight-streaming kernels (NT up to 48 rows, NN up to
+    16, cgvae_dense_pair_fwd), the column-per-thread gemm_skinny_kernel (NT, <= 16 rows, N >= 1024, where the streaming
+    kernel declines), SIMT cluster split-K (grid.z = S) and SIMT workspace split-K + splitk_reduce_kernel (TN);
   * colsum_tall_kernel from 4096 rows, rows split over a cluster of S = 8 / 4 / 1 CTAs (grid.y);
-  * the rank-segmented grouped weight gradient (data-parallel factor exchange).
+  * the rank-segmented grouped weight gradient (data-parallel factor exchange);
+  * the message-layer forward: message_fwd_kernel (SIMT) and message_tc_fwd_kernel (tensor cores, RC = 8).
 
 Every output is pre-filled with NaN (an element nobody writes fails), every case runs twice and must be bitwise repeatable.
 Metric: tests.golden_util.rel_err (max|a - b| / max|b|), evaluated on the device."""
@@ -27,7 +31,7 @@ import pytest
 import torch
 
 import coarsegrainingvae_b200 as cg
-from coarsegrainingvae_b200 import ops
+from coarsegrainingvae_b200 import ops, synthetic
 from oracle import cgvae_oracle as orc
 from tests import parity_cases as pc
 from tests.emulator import _act, _dact
@@ -56,7 +60,7 @@ def _base_name(name):
 
 
 def _probe(fn):
-    """run fn() under torch.profiler with CUDA activities; returns (fn's result, [(kernel base name, (gx, gy, gz))]) for
+    """run fn() under torch.profiler with CUDA activities; returns (fn's result, [(kernel base name, grid, block)]) for
     the kernels of this library (namespace cgvae), in launch order -- torch's own kernels (tensor set-up, a launch still
     draining when the profile starts) are left out.  A profile without kernel events fails: a path check that cannot see
     the kernels proves nothing."""
@@ -72,11 +76,11 @@ def _probe(fn):
             events = json.load(f).get("traceEvents", [])
     kernels = sorted((e for e in events if e.get("cat") == "kernel"), key=lambda e: e.get("ts", 0))
     assert kernels, "the profile holds no CUDA kernel events: the kernel this case must reach cannot be confirmed"
-    return result, [(_base_name(e["name"]), tuple(e.get("args", {}).get("grid", ()))) for e in kernels
-                    if "cgvae::" in e["name"]]
+    return result, [(_base_name(e["name"]), tuple(e.get("args", {}).get("grid", ())), tuple(e.get("args", {}).get("block", ())))
+                    for e in kernels if "cgvae::" in e["name"]]
 
 
-# expected launches per path: [(kernel, {grid axis: extent})]
+# expected launches per path: [(kernel, {grid axis: extent}[, block.x])]
 def _want(path):
     kind = path[0]
     if kind == "persistent":
@@ -87,15 +91,25 @@ def _want(path):
         return [("gemm_tc_kernel", {2: 8 * path[1]}), ("splitk_reduce_kernel", {})]
     if kind == "simt":
         return [("gemm_kernel", {2: 1})]
+    # (kind, grid, block): the whole launch shape is pinned
+    grid = dict(enumerate(path[1]))
+    if kind == "simt_cluster":                              # K split over a cluster of grid.z CTAs, reduced through DSMEM
+        return [("gemm_kernel", grid, path[2])]
+    if kind == "simt_splitk":                               # grid.z partial matrices, added in order by the reduce kernel
+        return [("gemm_kernel", grid, path[2]), ("splitk_reduce_kernel", {})]
+    if kind in ("gemm_skinny_kernel", "gemm_nt_stream_kernel", "gemm_nn_stream_kernel"):
+        return [(kind, grid, path[2])]
     raise ValueError(path)
 
 
 def _assert_launches(launches, want):
-    names = [n for n, _ in launches]
-    assert names == [n for n, _ in want], (launches, want)
-    for (name, grid), (_, axes) in zip(launches, want):
+    """launches: [(name, grid[, block])]; want: [(name, {grid axis: extent}[, block.x])]"""
+    assert [k[0] for k in launches] == [w[0] for w in want], (launches, want)
+    for (name, grid, *block), (_, axes, *blk) in zip(launches, want):
         for axis, extent in axes.items():
             assert grid[axis] == extent, (name, grid, axes)
+        if blk:
+            assert block[0][0] == blk[0], (name, block, blk)
 
 
 # ------------------------------------------------------------------------------------------ GEMM cases
@@ -138,9 +152,10 @@ def _nan_out(M, N, kind):
     return out, out
 
 
-def _poison_allocator(M, N):
-    """hand the caching allocator a NaN block of the pre-activation's size: a z_out the kernel does not write reads NaN."""
-    t = torch.full((M, N), NAN, device=DEV)
+def _poison_allocator(M, N, *shapes):
+    """hand the caching allocator NaN blocks of the pre-activation's size (and of `shapes`): a z_out the kernel does not
+    write reads NaN."""
+    t = [torch.full(s, NAN, device=DEV) for s in ((M, N),) + shapes]
     del t
 
 
@@ -261,6 +276,16 @@ GEMM_CASES = [
     ("simt_tn_ws_overflow", TN, 2048, 2048, 50000, ("simt",), dict()),                       # 3 x 16 MB partials > 32 MB
     ("simt_nt_misaligned_base", NT, 2000, 600, 600, ("simt",), dict(shift=1)),
     ("simt_nt_lda_not_4", NT, 2000, 600, 598, ("simt",), dict()),
+    # ---- fewer than 64 rows (decoder graphs: 12 beads, 36 vector rows), and the tcgen05 row threshold
+    ("skinny_nt_k100", NT, 12, 1024, 100, ("gemm_skinny_kernel", (16, 1, 2), 64), dict(bias=True, act=1)),   # K < 128
+    ("simt_cluster_nn_m36", NN, 36, 600, 600, ("simt_cluster", (19, 1, 5), 256), dict()),       # update-block mixes
+    ("simt_cluster_nt_m63", NT, 63, 256, 256, ("simt_cluster", (4, 1, 2), 256), dict()),
+    ("tc_cluster_nt_m64", NT, 64, 256, 256, ("cluster", 4), dict()),
+    ("simt_splitk_tn_m48", TN, 48, 600, 2000, ("simt_splitk", (10, 1, 16), 256), dict()),
+    ("stream_nt_m12", NT, 12, 600, 600, ("gemm_nt_stream_kernel", (75, 1, 1), 64), dict(bias=True, act=1)),
+    ("stream_nt_m36", NT, 36, 600, 600, ("gemm_nt_stream_kernel", (100, 1, 1), 128), dict(bias=True, act=1)),
+    ("stream_nn_m12", NN, 12, 600, 600, ("gemm_nn_stream_kernel", (10, 1, 8), 512), dict(dact=1)),
+    ("stream_nn_m12_s1", NN, 12, 19000, 256, ("gemm_nn_stream_kernel", (149, 1, 1), 512), dict()),    # cluster of one
 ]
 
 
@@ -268,6 +293,87 @@ GEMM_CASES = [
 def test_gemm_path_vs_float64(case):
     name, form, M, N, K, path, kw = case
     _gemm_case(form, M, N, K, path, seed=(M * 31 + N * 7 + K) % 100003, **kw)
+
+
+def test_linear_pair_adjacent_weights_one_stream_launch():
+    """ops.linear_pair_fwd with W1 / W2 adjacent in one buffer (u_mat / v_mat of an update block): one NT weight-streaming
+    launch over both weight matrices, each output against float64"""
+    M, N1, N2, K = 36, 600, 600, 600
+    gen = torch.Generator(device=DEV).manual_seed(36)
+    x = torch.randn(M, K, device=DEV, generator=gen)
+    W = torch.randn(N1 + N2, K, device=DEV, generator=gen) / math.sqrt(K)
+    W1, W2 = W[:N1], W[N1:]
+    _poison_allocator(M, N1, (M, N2))
+    (C1, C2), launches = _probe(lambda: ops.linear_pair_fwd(x, W1, W2))
+    _assert_launches(launches, [("gemm_nt_stream_kernel", {0: 120, 1: 1, 2: 1}, 256)])
+    for got, Wi in ((C1, W1), (C2, W2)):
+        err = _rel_err(got, _mm64(NT, x, Wi))
+        assert err < TOL, err
+    again = ops.linear_pair_fwd(x, W1, W2)
+    assert torch.equal(again[0], C1) and torch.equal(again[1], C2)
+
+
+# ------------------------------------------------------------------------------------------ message-layer forward
+
+def _message64(n_split, graph, geom, phi, v, Wf, bf, res_s, res_v):
+    """float64 message layer from the same per-edge records (basis, unit): conv.py:505-563 / 358-402"""
+    n, F = phi.shape[0], phi.shape[2]
+    E = int(graph.rowptr[-1])
+    col = graph.col.long()[:E]
+    recv = torch.repeat_interleave(torch.arange(n, device=DEV), (graph.rowptr[1:] - graph.rowptr[:-1]).long())[:E]
+    Wfull = torch.zeros(n_split * F, geom.rb, dtype=torch.float64, device=DEV)
+    Wfull[:, :geom.n_rbf] = Wf.double()
+    Wfull[:, geom.n_rbf] = bf.double()
+    m = phi.double()[col] * (geom.basis[:E].double() @ Wfull.t()).view(E, n_split, F)
+    dv_e = m[:, 2, None, :] * geom.unit[:E, :3].double()[:, :, None] + m[:, 0, None, :] * v.double()[col]
+    if n_split == 4:
+        dv_e = dv_e + m[:, 3, None, :] * torch.linalg.cross(v.double()[recv], v.double()[col], dim=1)
+    ds = torch.zeros(n, F, dtype=torch.float64, device=DEV).index_add_(0, recv, m[:, 1])
+    dv = torch.zeros(n, 3, F, dtype=torch.float64, device=DEV).index_add_(0, recv, dv_e)
+    return ds + res_s.double(), dv + res_v.double()
+
+
+# (n_split, MSG_TC, receivers, F, R, cutoff, expected launch (kernel, {grid axis: extent}, block.x))
+MESSAGE_CASES = [
+    ("simt_k3", 3, "0", 350, 600, 10, 12.0, ("message_fwd_kernel", {0: 88, 1: 19, 2: 1}, 128)),    # grid.x = ceil(350 / 4)
+    ("tc_k3_rc8", 3, "1", 350, 600, 10, 12.0, ("message_tc_fwd_kernel", {}, 320)),                  # 8 consumer warps
+    ("tc_k4_rc8", 4, "1", 250, 512, 8, 7.0, ("message_tc_fwd_kernel", {}, 320)),
+]
+
+
+@pytest.mark.parametrize("case", MESSAGE_CASES, ids=[c[0] for c in MESSAGE_CASES])
+def test_message_fwd_path_vs_float64(case):
+    _, n_split, tc, n, F, R, cutoff, want = case
+    gen = torch.Generator().manual_seed(n + F)
+    xyz = torch.as_tensor(synthetic.lattice_points(n, 2.2, np.random.default_rng(n), rotate=False), device=DEV)
+    half = ops.radius_graph(xyz, cutoff, True)
+    graph = ops.build_graph(torch.cat([half, half.flip(1)], 0), n)
+    geom = ops.edge_geometry(graph, xyz, xyz, R, cutoff)
+    phi = torch.randn(n, n_split, F, generator=gen).to(DEV)
+    v = torch.randn(n, 3, F, generator=gen).to(DEV)
+    Wf = (torch.randn(n_split * F, R, generator=gen) * 0.5).to(DEV)
+    bf = (torch.randn(n_split * F, generator=gen) * 0.5).to(DEV)
+    res_s, res_v = torch.randn(n, F, generator=gen).to(DEV), torch.randn(n, 3, F, generator=gen).to(DEV)
+    old = ops.MSG_TC, ops.MSG_TC_RC, ops.MSG_TC_CROSS_RC
+    try:
+        ops.MSG_TC, ops.MSG_TC_RC, ops.MSG_TC_CROSS_RC = tc, 8, 8
+        if tc == "1":
+            ops.message_tiles(geom, False, 8)               # built once per graph, outside the profiled call
+
+        def call():
+            _poison_allocator(n, F, (n, 3, F))
+            return ops.message_fwd(n_split, phi, v, v if n_split == 4 else None, geom, Wf, bf, res_s, res_v)
+
+        got, launches = _probe(call)
+        again = call()
+    finally:
+        ops.MSG_TC, ops.MSG_TC_RC, ops.MSG_TC_CROSS_RC = old
+    _assert_launches([k for k in launches if k[0] == want[0]], [want])
+    ds, dv = _message64(n_split, graph, geom, phi, v, Wf, bf, res_s, res_v)
+    for a, b in ((got[0], ds), (got[1], dv)):
+        err = _rel_err(a, b)
+        assert err < TOL, err
+    assert torch.equal(again[0], got[0]) and torch.equal(again[1], got[1])
 
 
 # ------------------------------------------------------------------------------------------ column sums
@@ -428,13 +534,14 @@ def test_update_block_c4_size_vs_float64(paired):
     ds, dv = blk(s, v)
     loss = (ds * gs).sum() + (dv * gv).sum()
     _, launches = _probe(loss.backward)
-    names = [k for k, _ in launches]
-    assert ("gemm_tc_persistent_kernel", (NUM_SM, 1, 1)) in launches, launches
+    names = [k for k, _, _ in launches]
+    grids = [(k, g) for k, g, _ in launches]
+    assert ("gemm_tc_persistent_kernel", (NUM_SM, 1, 1)) in grids, launches
     assert "colsum_tall_kernel" in names, launches
-    grouped = [i for i, (k, g) in enumerate(launches) if k == "gemm_tc_kernel" and g[2] == 16]
+    grouped = [i for i, (k, g) in enumerate(grids) if k == "gemm_tc_kernel" and g[2] == 16]
     assert grouped and "splitk_reduce_kernel" in names[grouped[0]:], launches
     if paired:      # [gU; gV] over 48 000 rows as ONE [1024, 512] contraction (4 x 8 tiles, 2 groups of 8)
-        assert ("gemm_tc_kernel", (4, 8, 16)) in launches, launches
+        assert ("gemm_tc_kernel", (4, 8, 16)) in grids, launches
     # oracle: fp32 (for the conditioning-aware criterion) and float64 (the truth), both on the device
     outs = {}
     for dt in (torch.float32, torch.float64):

@@ -232,7 +232,7 @@ def _gemm_tf32_case(form, M, N, K, path, seed, bias=False, act=0, z_out=False, d
 
 def _tc_cases():
     dp = _gemm_setup()
-    return [c for c in dp.GEMM_CASES if c[5][0] != "simt"]
+    return [c for c in dp.GEMM_CASES if c[5][0] in ("persistent", "cluster", "grouped")]
 
 
 TC_CASES = _tc_cases()

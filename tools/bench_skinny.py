@@ -23,7 +23,6 @@ def bench(fn_list, iters=5):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / (iters * len(fn_list)) * 1e3
 shapes = [("W1", 600, 600), ("W2", 5400, 600), ("A0", 600, 1200), ("A1", 1800, 600)]
-print("env skinny=%s cluster=%s" % (os.environ.get("CGVAE_SKINNY_GEMM", "1"), os.environ.get("CGVAE_CLUSTER_SPLITK", "1")))
 for M in (12, 36):
     for name, n_out, n_in in shapes:
         nbuf = max(2, int(300e6 // (n_out * n_in * 4)))

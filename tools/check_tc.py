@@ -1,5 +1,5 @@
 """tcgen05 3xTF32 GEMM (csrc/gemm_tc.cu) vs float64, all operand forms, timed inside a CUDA graph (20 launches per replay,
-operands rotated through 4 buffers); run with CGVAE_TCGEN05=0 for the fp32 SIMT tiles on the same shapes.
+operands rotated through 4 buffers).
     python tools/check_tc.py [--big]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -26,7 +26,6 @@ shapes = [(350, 1800, 600), (350, 600, 600), (350, 600, 1800), (704, 600, 600), 
           (4000, 2048, 512)]
 if "--big" in sys.argv:
     shapes += [(16000, 2048, 512), (128000, 600, 600)]
-print("tcgen05 enabled:", os.environ.get("CGVAE_TCGEN05", "1"))
 for (M, N, K) in shapes:
     g = torch.Generator().manual_seed(M + N)
     A = torch.randn(M, K, generator=g); W = torch.randn(N, K, generator=g) / K ** 0.5; b = torch.randn(N, generator=g)

@@ -27,6 +27,5 @@ for k, p in model.named_parameters():
     if P[k].grad is None or p.grad is None or float(P[k].grad.abs().max()) == 0: continue
     rows.append((rel_err(p.grad, P[k].grad), rel_err(p.grad, P64[k].grad), rel_err(P[k].grad, P64[k].grad), k))
 rows.sort(reverse=True)
-print("tcgen05:", os.environ.get("CGVAE_TCGEN05", "1"))
 print("%-12s %-12s %-12s %s" % ("kern-vs-f32", "kern-vs-f64", "f32-vs-f64", "tensor"))
 for r in rows[:6]: print("%-12.3e %-12.3e %-12.3e %s" % r)
