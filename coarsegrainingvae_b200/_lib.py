@@ -37,6 +37,8 @@ SIGNATURES = {
     "cgvae_segment_count": (_INT, [_P, _I64, _I64, _P, _P]),
     "cgvae_segment_rank": (_INT, [_P, _I64, _I64, _P, _P, _P, _P, _P, _P]),
     "cgvae_edge_geometry": (_INT, [_P, _P, _P, _P, _P, _I64, _I64, _P, _INT, _INT, _F32, _P, _P, _P, _P, _P]),
+    "cgvae_edge_geometry_bwd": (_INT, [_P, _P, _P, _P, _P, _I64, _I64, _P, _INT, _INT, _F32, _P, _P, _P, _P, _P, _P]),
+    "cgvae_edge_coord_reduce": (_INT, [_P, _P, _I64, _P, _P, _I64, _INT, _P, _P, _P]),
     "cgvae_gemm": (_INT, [_INT, _P, _I64, _P, _I64, _P, _I64, _I64, _I64, _I64, _P, _INT, _P, _P, _INT, _P, _P, _SZ, _P, _INT, _P]),
     "cgvae_dense_pair_fwd": (_INT, [_P, _I64, _P, _I64, _I64, _I64, _I64, _I64, _P, _P, _P]),
     "cgvae_colsum": (_INT, [_P, _I64, _I64, _I64, _P, _P]),
@@ -46,6 +48,8 @@ SIGNATURES = {
     "cgvae_message_bwd_ws_bytes": (_SZ, [_INT, _INT, _INT, _I64]),
     "cgvae_message_bwd": (_INT, [_INT, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _INT, _INT, _INT, _P, _P,
                                  _INT, _INT, _P, _P, _P, _P, _P, _SZ, _P]),
+    "cgvae_message_geom_bwd": (_INT, [_INT, _P, _P, _P, _P, _P, _I64, _I64, _P, _P, _P, _P, _INT, _INT, _INT, _P, _P, _INT, _P,
+                                      _P, _P]),
     "cgvae_msg_tiles_batches_cap": (_I64, [_I64, _I64, _I64, _INT]),
     "cgvae_msg_tiles_rec_bytes": (_SZ, []),
     "cgvae_msg_tiles_build": (_INT, [_P, _P, _P, _I64, _I64, _I64, _P, _P, _INT, _INT, _P, _P, _P, _P, _I64, _P]),
@@ -87,6 +91,7 @@ SIGNATURES = {
     "cgvae_loss_ws_bytes": (_SZ, []),
     "cgvae_loss_fwd": (_INT, [_P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _INT, _P, _F32, _F32, _P, _P, _SZ, _P]),
     "cgvae_loss_bwd": (_INT, [_P, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _I64, _INT, _P, _F32, _F32, _P, _P, _P, _P, _P, _P]),
+    "cgvae_loss_bwd_target": (_INT, [_P, _P, _P, _I64, _P, _P, _P, _F32, _P, _P]),
     "cgvae_fill": (_INT, [_P, _I64, _F32, _P]),
     "cgvae_vec_to_planar": (_INT, [_P, _I64, _INT, _P, _P]),
     "cgvae_vec_from_planar": (_INT, [_P, _I64, _INT, _P, _P]),

@@ -50,7 +50,7 @@ class BatchGraphs(object):
     def geometry(self, which, xyz_send, xyz_recv, n_rbf, cutoff):
         key = (which, int(n_rbf), float(cutoff))
         if key not in self._geom:
-            self._geom[key] = ops.edge_geometry(getattr(self, which), xyz_send, xyz_recv, n_rbf, cutoff)
+            self._geom[key] = fn.edge_geometry(getattr(self, which), xyz_send, xyz_recv, n_rbf, cutoff)
         return self._geom[key]
 
 

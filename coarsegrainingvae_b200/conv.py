@@ -32,7 +32,7 @@ def to_module(activation):
 
 def _geometry_from_edges(nbrs, r_ij, n_nodes, n_rbf, cutoff, edge_wgt=None):
     graph = ops.build_graph(nbrs, n_nodes)
-    return ops.edge_geometry(graph, None, None, n_rbf, cutoff, edge_wgt=edge_wgt, r_edge=r_ij)
+    return fn.edge_geometry(graph, None, None, n_rbf, cutoff, edge_wgt=edge_wgt, r_edge=r_ij)
 
 
 class InvariantMessage(nn.Module):
@@ -67,13 +67,13 @@ class _MessageBase(nn.Module):
     def fused(self, s, v, geom):
         """(s, v) + message, planar layout; v may be None (all zero)."""
         return fn.MessageBlock.apply(geom, self.n_split, "self", self.inv_message.act, s, v, None, None,
-                                     *self.inv_message.params())
+                                     *self.inv_message.params(), geom.basis, geom.unit)
 
     def forward(self, s_j, v_j, r_ij, nbrs, edge_wgt=None):
         geom = _geometry_from_edges(nbrs, r_ij, s_j.shape[0], self.inv_message.n_rbf, self.inv_message.cutoff, edge_wgt)
         # the layout conversions [N,F,3] <-> [N,3,F] are autograd nodes of their own
         ds, dv = fn.MessageBlock.apply(geom, self.n_split, "delta", self.inv_message.act, s_j, _Planar.apply(v_j), None, None,
-                                       *self.inv_message.params())
+                                       *self.inv_message.params(), geom.basis, geom.unit)
         return ds, _Unplanar.apply(dv)
 
 
@@ -128,13 +128,14 @@ class EquiMessagePsuedo(nn.Module):
                                             n_rbf=n_rbf, cutoff=cutoff, dropout=dropout)
 
     def fused(self, s, sbar, v, vbar, geom):
-        return fn.Message9Block.apply(geom, True, self.inv_message.act, s, sbar, v, vbar, *self.inv_message.params())
+        return fn.Message9Block.apply(geom, True, self.inv_message.act, s, sbar, v, vbar, *self.inv_message.params(),
+                                      geom.basis, geom.unit)
 
     def forward(self, s_j, sbar_j, v_j, vbar_j, r_ij, nbrs, edge_wgt=None):
         # edge_wgt is accepted and ignored, exactly like the reference (conv.py:180-187 never reads it)
         geom = _geometry_from_edges(nbrs, r_ij, s_j.shape[0], self.inv_message.n_rbf, self.inv_message.cutoff)
         ds, dsbar, dv, dvbar = fn.Message9Block.apply(geom, False, self.inv_message.act, s_j, sbar_j, _Planar.apply(v_j), _Planar.apply(vbar_j),
-                                                      *self.inv_message.params())
+                                                      *self.inv_message.params(), geom.basis, geom.unit)
         return ds, dsbar, _Unplanar.apply(dv), _Unplanar.apply(dvbar)
 
 
@@ -199,7 +200,7 @@ class ContractiveMessageBlock(nn.Module):
 
     def fused(self, s, v, H, V, geom):
         """(H, V) + contraction of atom state (s, v) over the atoms->beads graph."""
-        return fn.MessageBlock.apply(geom, 3, "other", self.act, s, v, H, V, *self.params())
+        return fn.MessageBlock.apply(geom, 3, "other", self.act, s, v, H, V, *self.params(), geom.basis, geom.unit)
 
     def forward(self, s_i, v_i, r_iI, mapping):
         # scatter_add without dim_size (conv.py:725-731): the output has max(mapping)+1 rows -- one host read,
@@ -207,6 +208,7 @@ class ContractiveMessageBlock(nn.Module):
         n_beads = int(mapping.max().item()) + 1
         seg = ops.build_segments(mapping, n_beads)
         graph = ops.contraction_graph(seg)
-        geom = ops.edge_geometry(graph, None, None, self.n_rbf, self.cutoff, r_edge=r_iI)
-        dS, dV = fn.MessageBlock.apply(geom, 3, "delta", self.act, s_i, _Planar.apply(v_i), None, None, *self.params())
+        geom = fn.edge_geometry(graph, None, None, self.n_rbf, self.cutoff, r_edge=r_iI)
+        dS, dV = fn.MessageBlock.apply(geom, 3, "delta", self.act, s_i, _Planar.apply(v_i), None, None, *self.params(),
+                                       geom.basis, geom.unit)
         return dS, _Unplanar.apply(dV)

@@ -151,6 +151,24 @@ __device__ __forceinline__ float warp_sum(float x) {
   return x;
 }
 
+// receiver of CSR slot `slot`: the largest row with rowptr[row] <= slot
+__device__ __forceinline__ int row_of_slot(const int32_t* __restrict__ rowptr, int64_t n_rows, int slot) {
+  int64_t lo = 0, hi = n_rows;
+  while (hi - lo > 1) {
+    const int64_t mid = (lo + hi) >> 1;
+    if (rowptr[mid] <= slot) lo = mid; else hi = mid;
+  }
+  return (int)lo;
+}
+
+// message filter column for (split k, channel f): rows r < R from Wf[(k*F+f)][r], row R = bias, rest zero
+__device__ __forceinline__ float filter_entry(const float* __restrict__ Wf, const float* __restrict__ bf, int F, int R,
+                                              int k, int f, int r) {
+  if (r < R) return Wf[((int64_t)k * F + f) * R + r];
+  if (r == R) return bf[(int64_t)k * F + f];
+  return 0.f;
+}
+
 __device__ __forceinline__ float swish_f(float z) { return z / (1.0f + expf(-z)); }
 // d/dz [z * sigmoid(z)] = sig * (1 + z * (1 - sig))
 __device__ __forceinline__ float dswish_f(float z) {

@@ -4,15 +4,6 @@
 
 namespace cgvae {
 
-__device__ __forceinline__ int row_of_slot(const int32_t* __restrict__ rowptr, int64_t n_rows, int slot) {
-  int64_t lo = 0, hi = n_rows;  // largest row with rowptr[row] <= slot
-  while (hi - lo > 1) {
-    const int64_t mid = (lo + hi) >> 1;
-    if (rowptr[mid] <= slot) lo = mid; else hi = mid;
-  }
-  return (int)lo;
-}
-
 __global__ void __launch_bounds__(256) edge_geometry_kernel(
     const float* __restrict__ xs, const float* __restrict__ xr, const float* __restrict__ r_edge,
     const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, int64_t n_recv, int64_t E,
@@ -76,6 +67,100 @@ __global__ void __launch_bounds__(256) edge_geometry_kernel(
   }
 }
 
+// Backward of edge_geometry_kernel, the autograd of the reference's expressions (conv.py:25-29, modules.py:52-58,148-172):
+//   d = sqrt(sum_c (r_c^2 + 1e-8)), dd/dr = u;  rbf_n' = (c_n cos(c_n d) - sin(c_n d) / d) / d;
+//   env' = -1/2 (pi / cutoff) sin(pi d / cutoff); basis derivatives vanish for d >= cutoff; edge_wgt multiplies;
+//   dr = dd u + (du - <u, du> u) / d.
+// d_basis / d_unit (nullable = zero) are the cotangents of basis / unit.  Writes dr[e] per CSR slot (padded tail slots of a
+// static-capacity graph: zero), or, with r_edge, d_r_edge[eid[e]] (every original edge owns exactly one slot).
+__global__ void __launch_bounds__(256) edge_geometry_bwd_kernel(
+    const float* __restrict__ xs, const float* __restrict__ xr, const float* __restrict__ r_edge,
+    const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col, int64_t n_recv, int64_t E,
+    const float* __restrict__ coef, int R, int RB, float cutoff, const float* __restrict__ edge_wgt, const int32_t* __restrict__ eid,
+    const float* __restrict__ d_basis, const float* __restrict__ d_unit, float* __restrict__ dr) {
+  CGVAE_KERNEL_PROLOGUE();
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= E) return;
+  const int64_t o = (r_edge != nullptr && eid != nullptr) ? eid[e] : e;
+  if (e >= rowptr[n_recv]) {
+    dr[o * 3 + 0] = 0.f; dr[o * 3 + 1] = 0.f; dr[o * 3 + 2] = 0.f;
+    return;
+  }
+  float rx, ry, rz;
+  if (r_edge != nullptr) {
+    rx = r_edge[o * 3 + 0]; ry = r_edge[o * 3 + 1]; rz = r_edge[o * 3 + 2];
+  } else {
+    const int i = row_of_slot(rowptr, n_recv, (int)e);
+    const int j = col[e];
+    rx = xs[(int64_t)j * 3 + 0] - xr[(int64_t)i * 3 + 0];
+    ry = xs[(int64_t)j * 3 + 1] - xr[(int64_t)i * 3 + 1];
+    rz = xs[(int64_t)j * 3 + 2] - xr[(int64_t)i * 3 + 2];
+  }
+  const float d = sqrtf((rx * rx + 1e-8f) + (ry * ry + 1e-8f) + (rz * rz + 1e-8f));
+  const float ux = rx / d, uy = ry / d, uz = rz / d;
+  float gd = 0.f, gux = 0.f, guy = 0.f, guz = 0.f;
+  if (d_unit != nullptr) {
+    const float4 g = reinterpret_cast<const float4*>(d_unit)[e];
+    gux = g.x; guy = g.y; guz = g.z; gd = g.w;
+  }
+  if (d_basis != nullptr && d < cutoff) {
+    const float wgt = edge_wgt != nullptr ? edge_wgt[eid ? eid[e] : e] : 1.0f;
+    const float a = 3.14159265358979323846f / cutoff;
+    const float env = 0.5f * (cosf(a * d) + 1.0f);
+    const float denv = -0.5f * a * sinf(a * d);
+    const float* gb = d_basis + e * RB;
+    float acc = gb[R] * denv;
+    for (int r = 0; r < R; ++r) {
+      const float c = coef[r];
+      float sn, cs;
+      sincosf(c * d, &sn, &cs);
+      const float rbf = sn / d;
+      const float drbf = (c * cs - rbf) / d;
+      acc = fmaf(gb[r], fmaf(drbf, env, rbf * denv), acc);
+    }
+    gd = fmaf(acc, wgt, gd);
+  }
+  const float ug = ux * gux + uy * guy + uz * guz;
+  dr[o * 3 + 0] = fmaf(gd, ux, (gux - ug * ux) / d);
+  dr[o * 3 + 1] = fmaf(gd, uy, (guy - ug * uy) / d);
+  dr[o * 3 + 2] = fmaf(gd, uz, (guz - ug * uz) / d);
+}
+
+// Coordinate gradients from the per-slot dr (r_e = x_send[j] - x_recv[i]): g_send[j] = sum of dr over the sender CSR row,
+// g_recv[i] = -sum of dr over the receiver CSR row, each in CSR order.  same != 0 (one node set, one coordinate tensor):
+// g_send[n] = send sum - receive sum, g_recv unused.
+__global__ void __launch_bounds__(256) edge_coord_reduce_kernel(
+    const float* __restrict__ dr, const int32_t* __restrict__ rowptr, int64_t n_recv, const int32_t* __restrict__ rowptr_t,
+    const int32_t* __restrict__ perm_t, int64_t n_send, int same, float* __restrict__ g_send, float* __restrict__ g_recv) {
+  CGVAE_KERNEL_PROLOGUE();
+  const int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  float sx = 0.f, sy = 0.f, sz = 0.f;
+  if (n < n_send) {
+    for (int t = rowptr_t[n]; t < rowptr_t[n + 1]; ++t) {
+      const int64_t e = perm_t[t];
+      sx += dr[e * 3 + 0]; sy += dr[e * 3 + 1]; sz += dr[e * 3 + 2];
+    }
+  }
+  float qx = 0.f, qy = 0.f, qz = 0.f;
+  if (n < n_recv) {
+    for (int e = rowptr[n]; e < rowptr[n + 1]; ++e) {
+      qx += dr[(int64_t)e * 3 + 0]; qy += dr[(int64_t)e * 3 + 1]; qz += dr[(int64_t)e * 3 + 2];
+    }
+  }
+  if (same) {
+    if (n < n_send) {
+      g_send[n * 3 + 0] = sx - qx; g_send[n * 3 + 1] = sy - qy; g_send[n * 3 + 2] = sz - qz;
+    }
+    return;
+  }
+  if (n < n_send) {
+    g_send[n * 3 + 0] = sx; g_send[n * 3 + 1] = sy; g_send[n * 3 + 2] = sz;
+  }
+  if (n < n_recv) {
+    g_recv[n * 3 + 0] = -qx; g_recv[n * 3 + 1] = -qy; g_recv[n * 3 + 2] = -qz;
+  }
+}
+
 // reference layout v[N][F][3] <-> planar v[N][3][F]
 __global__ void vec_to_planar_kernel(const float* __restrict__ in, int64_t N, int F, float* __restrict__ out) {
   CGVAE_KERNEL_PROLOGUE();
@@ -112,6 +197,33 @@ int cgvae_edge_geometry(const float* xyz_send, const float* xyz_recv, const floa
   launch_kernel(edge_geometry_kernel, dim3((unsigned)ceil_div(n_edges, 256)), dim3(256), 0, (cudaStream_t)stream, 
       xyz_send, xyz_recv, r_edge, rowptr, col, n_recv, n_edges, coef, R, RB, cutoff, edge_wgt, eid, basis, unit);
   return launched("edge_geometry");
+}
+
+int cgvae_edge_geometry_bwd(const float* xyz_send, const float* xyz_recv, const float* r_edge, const int32_t* rowptr,
+                            const int32_t* col, int64_t n_recv, int64_t n_edges, const float* coef, int R, int RB, float cutoff,
+                            const float* edge_wgt, const int32_t* eid, const float* d_basis, const float* d_unit, float* dr,
+                            cgvae_stream_t stream) {
+  if (n_edges == 0) return 0;
+  CGVAE_REQUIRE(((xyz_send && xyz_recv) || r_edge) && rowptr && col && coef && dr && (r_edge == nullptr || eid),
+                "edge_geometry_bwd: null pointer");
+  CGVAE_REQUIRE(R >= 1 && RB >= R + 1 && (RB % 4) == 0, "edge_geometry_bwd: need RB %% 4 == 0 and RB >= R+1 (R=%d RB=%d)", R, RB);
+  CGVAE_REQUIRE(d_unit == nullptr || aligned16(d_unit), "edge_geometry_bwd: d_unit must be 16-byte aligned");
+  launch_kernel(edge_geometry_bwd_kernel, dim3((unsigned)ceil_div(n_edges, 256)), dim3(256), 0, (cudaStream_t)stream, xyz_send,
+                xyz_recv, r_edge, rowptr, col, n_recv, n_edges, coef, R, RB, cutoff, edge_wgt, eid, d_basis, d_unit, dr);
+  return launched("edge_geometry_bwd");
+}
+
+int cgvae_edge_coord_reduce(const float* dr, const int32_t* rowptr, int64_t n_recv, const int32_t* rowptr_t,
+                            const int32_t* perm_t, int64_t n_send, int same, float* g_send, float* g_recv,
+                            cgvae_stream_t stream) {
+  CGVAE_REQUIRE(!same || n_recv == n_send, "edge_coord_reduce: same needs one node set (n_recv=%lld n_send=%lld)",
+                (long long)n_recv, (long long)n_send);
+  const int64_t n = std::max(n_recv, n_send);
+  if (n == 0) return 0;
+  CGVAE_REQUIRE(dr && rowptr && rowptr_t && perm_t && g_send && (same || g_recv), "edge_coord_reduce: null pointer");
+  launch_kernel(edge_coord_reduce_kernel, dim3((unsigned)ceil_div(n, 256)), dim3(256), 0, (cudaStream_t)stream, dr, rowptr, n_recv,
+                rowptr_t, perm_t, n_send, same, g_send, g_recv);
+  return launched("edge_coord_reduce");
 }
 
 int cgvae_vec_to_planar(const float* v_nf3, int64_t N, int F, float* v_n3f, cgvae_stream_t stream) {

@@ -185,6 +185,41 @@ __global__ void __launch_bounds__(256) loss_bwd_xyz_kernel(const float* __restri
   g_rec[3 * a + 2] = g * gz;
 }
 
+// gradient to the TARGET coordinates (xyz is also the encoder input when coordinates are differentiated):
+// g_xyz[a] = g * ( -2 (x_rec_a - x_a) / (3 n_atoms) - gamma / n_bonds * sum_b 2 (gen - dat) / dat * (x_a - x_b) )
+__global__ void __launch_bounds__(256) loss_bwd_target_kernel(const float* __restrict__ g_loss, const float* __restrict__ xyz,
+                                                              const float* __restrict__ xyz_rec, int64_t n_atoms,
+                                                              const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                                                              const float* __restrict__ norms, float gamma, float* __restrict__ g_xyz) {
+  CGVAE_KERNEL_PROLOGUE();
+  const int64_t a = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (a >= n_atoms) return;
+  const float g = g_loss[0];
+  const float n_at = norms ? norms[0] : (float)n_atoms;
+  const float xa = xyz[3 * a], ya = xyz[3 * a + 1], za = xyz[3 * a + 2];
+  const float xr = xyz_rec[3 * a], yr = xyz_rec[3 * a + 1], zr = xyz_rec[3 * a + 2];
+  const float cr = 2.0f / (3.0f * n_at);
+  float gx = cr * (xa - xr), gy = cr * (ya - yr), gz = cr * (za - zr);
+  if (rowptr != nullptr && gamma != 0.f) {
+    const float n_bo = norms ? norms[2] : 0.5f * (float)rowptr[n_atoms];
+    const float cb = gamma / fmaxf(n_bo, 1e-30f);
+    float bx = 0.f, by = 0.f, bz = 0.f;
+    for (int t = rowptr[a]; t < rowptr[a + 1]; ++t) {
+      const int64_t b = col[t];
+      const float dx = xr - xyz_rec[3 * b], dy = yr - xyz_rec[3 * b + 1], dz = zr - xyz_rec[3 * b + 2];
+      const float ex = xa - xyz[3 * b], ey = ya - xyz[3 * b + 1], ez = za - xyz[3 * b + 2];
+      const float gen = sqrtf(dx * dx + dy * dy + dz * dz + kBondEps);
+      const float dat = sqrtf(ex * ex + ey * ey + ez * ez + kBondEps);
+      const float k = 2.0f * (dat - gen) / dat;
+      bx = fmaf(k, ex, bx); by = fmaf(k, ey, by); bz = fmaf(k, ez, bz);
+    }
+    gx = fmaf(cb, bx, gx); gy = fmaf(cb, by, gy); gz = fmaf(cb, bz, gz);
+  }
+  g_xyz[3 * a] = g * gx;
+  g_xyz[3 * a + 1] = g * gy;
+  g_xyz[3 * a + 2] = g * gz;
+}
+
 // gradients of beta * KL to (mu, sigma, prior mean, prior std)
 __global__ void __launch_bounds__(256) loss_bwd_kl_kernel(const float* __restrict__ g_loss, const float* __restrict__ mu,
                                                           const float* __restrict__ sigma, const float* __restrict__ pmu,
@@ -400,6 +435,14 @@ int cgvae_loss_bwd(const float* g_loss, const float* xyz, const float* xyz_rec, 
 
 /* Dihedral loss (scripts/pcn_utils.py:114-132,178-180): out[0] = mean_d (theta(rec; idx[d]) - theta(xyz; idx[d]))^2.
  * contrib [n_dihe][4][3]: unscaled per-(dihedral, slot) gradients kept for the backward; ws: 256 floats. */
+int cgvae_loss_bwd_target(const float* g_loss, const float* xyz, const float* xyz_rec, int64_t n_atoms, const int32_t* bond_rowptr,
+                          const int32_t* bond_col, const float* norms, float gamma, float* g_xyz, cgvae_stream_t stream) {
+  CGVAE_REQUIRE(g_loss && xyz && xyz_rec && g_xyz && n_atoms > 0, "loss_bwd_target: null pointer / no atoms");
+  launch_kernel(loss_bwd_target_kernel, dim3((unsigned)ceil_div(n_atoms, 256)), dim3(256), 0, (cudaStream_t)stream, g_loss, xyz,
+                xyz_rec, n_atoms, bond_rowptr, bond_col, norms, gamma, g_xyz);
+  return launched("loss_bwd_target");
+}
+
 int cgvae_dihedral_loss_fwd(const float* xyz, const float* xyz_rec, const int64_t* idx, int64_t n_dihe, const int64_t* n_live,
                             const float* norm, float* contrib, float* out, void* ws, size_t ws_bytes, cgvae_stream_t stream) {
   cudaStream_t st = (cudaStream_t)stream;

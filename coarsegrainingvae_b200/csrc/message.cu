@@ -24,14 +24,6 @@ __device__ __forceinline__ void load_basis(const float* __restrict__ basis, int 
   }
 }
 
-// filter column for (split k, channel f): rows r < R from Wf[(k*F+f)][r], row R = bias, rest zero
-__device__ __forceinline__ float filter_entry(const float* __restrict__ Wf, const float* __restrict__ bf, int F, int R,
-                                              int k, int f, int r) {
-  if (r < R) return Wf[((int64_t)k * F + f) * R + r];
-  if (r == R) return bf[(int64_t)k * F + f];
-  return 0.f;
-}
-
 // ------------------------------------------------------------------------------------------
 // forward, 3 or 4 splits
 // ------------------------------------------------------------------------------------------

@@ -1,6 +1,8 @@
 """Autograd nodes of the hot path: every forward and every backward is a short sequence of C-ABI
 kernel launches (ops.py); PyTorch only owns memory and the tape.  Gradients flow to features and
-parameters, never to coordinates (geometry comes from data: cgvae.py:276-280, SURVEY.md section 7).
+parameters, and to atom / bead coordinates (or the r_ij of the block API) when one of them requires
+grad: the edge geometry then becomes an EdgeGeometry node and the message layers also return the
+cotangents of its basis / unit records (DESIGN.md section 4).
 
 Backward formulas: SURVEY.md Appendix A (checked against the oracle's autograd in tests/).
 """
@@ -78,6 +80,47 @@ class LinearFn(Function):
         return gx, gW, gb
 
 
+def _requires_grad(*tensors):
+    return torch.is_grad_enabled() and any(t is not None and t.requires_grad for t in tensors)
+
+
+class EdgeGeometry(Function):
+    """ops.edge_geometry as an autograd node (same launch, same bits); backward = the geometry backward plus the node
+    reductions to the sender / receiver coordinates, or the gradient of r_edge.  xyz_recv None: one coordinate tensor
+    for both ends of every edge (atom graph, CG graph)."""
+
+    @staticmethod
+    def forward(ctx, graph, n_rbf, cutoff, xyz_send, xyz_recv, r_edge, edge_wgt):
+        same = xyz_send is not None and xyz_recv is None
+        geom = ops.edge_geometry(graph, xyz_send, xyz_send if same else xyz_recv, n_rbf, cutoff, edge_wgt=edge_wgt, r_edge=r_edge)
+        ctx.graph, ctx.n_rbf, ctx.cutoff, ctx.same = graph, n_rbf, cutoff, same     # not geom: it holds the outputs
+        ctx.save_for_backward(xyz_send, xyz_recv, r_edge, edge_wgt)
+        return geom.basis, geom.unit
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, d_basis, d_unit):
+        xyz_send, xyz_recv, r_edge, edge_wgt = ctx.saved_tensors
+        if ctx.needs_input_grad[6]:
+            raise NotImplementedError("coordinate gradients: the gradient to edge_wgt is not implemented")
+        dr = ops.edge_geometry_bwd(ctx.graph, ctx.n_rbf, ctx.cutoff, xyz_send, xyz_send if ctx.same else xyz_recv, d_basis, d_unit,
+                                   edge_wgt, r_edge)
+        if r_edge is not None:
+            return None, None, None, None, None, dr, None
+        g_send, g_recv = ops.edge_coord_reduce(ctx.graph, dr, ctx.same)
+        return None, None, None, g_send, g_recv, None, None
+
+
+def edge_geometry(graph, xyz_send, xyz_recv, n_rbf, cutoff, edge_wgt=None, r_edge=None):
+    """ops.edge_geometry, differentiable when grad mode is on and a coordinate, r_edge or edge_wgt requires grad (the
+    only case in which the geometry backward kernels run); otherwise the plain launch."""
+    if not _requires_grad(xyz_send, xyz_recv, r_edge, edge_wgt):
+        return ops.edge_geometry(graph, xyz_send, xyz_recv, n_rbf, cutoff, edge_wgt=edge_wgt, r_edge=r_edge)
+    same = xyz_send is xyz_recv
+    basis, unit = EdgeGeometry.apply(graph, n_rbf, cutoff, xyz_send, None if same else xyz_recv, r_edge, edge_wgt)
+    return ops.Geometry(graph, basis, unit, n_rbf, ops.rb_for(n_rbf), cutoff)
+
+
 class MessageBlock(Function):
     """InvariantMessage + EquiMessageBlock (n_split 3, conv.py:505-563) / EquiMessageCross (4, conv.py:358-402) /
     ContractiveMessageBlock (3 on the atoms->beads graph, conv.py:703-733).
@@ -86,10 +129,11 @@ class MessageBlock(Function):
     mode 'delta' : out = message            (the reference block API)
     mode 'other' : out = (res_s, res_v) + message, residual state on the receiver set (contraction)
     v None means v == 0 (first layer of every stack) and skips the vector gathers.
+    basis / unit are geom.basis / geom.unit, inputs so that their cotangents reach an EdgeGeometry node.
     """
 
     @staticmethod
-    def forward(ctx, geom, n_split, mode, act, s, v, res_s, res_v, W1, b1, W2, b2, Wf, bf):
+    def forward(ctx, geom, n_split, mode, act, s, v, res_s, res_v, W1, b1, W2, b2, Wf, bf, basis, unit):
         s = s.contiguous()
         a1, z1, phi = _phi_forward(s, W1, b1, W2, b2, act)
         N, F = s.shape
@@ -124,14 +168,17 @@ class MessageBlock(Function):
         gv = None if ctx.v_none else g_v_send
         g_res_s = g_s if mode == "other" else None
         g_res_v = g_v if (mode == "other" and not ctx.res_v_none) else None
-        return None, None, None, None, gs, gv, g_res_s, g_res_v, gW1, gb1, gW2, gb2, dWf, dbf
+        d_basis = d_unit = None
+        if ctx.needs_input_grad[14] or ctx.needs_input_grad[15]:
+            d_basis, d_unit = ops.message_geom_bwd(n_split, phi3, v, v if n_split == 4 else None, ctx.geom, Wf, bf, g_s, g_v)
+        return None, None, None, None, gs, gv, g_res_s, g_res_v, gW1, gb1, gW2, gb2, dWf, dbf, d_basis, d_unit
 
 
 class Message9Block(Function):
     """InvariantMessage (9 splits) + EquiMessagePsuedo, conv.py:180-242; residual adds of cgvae.py:108-111 fused."""
 
     @staticmethod
-    def forward(ctx, geom, residual, act, s, sbar, v, vbar, W1, b1, W2, b2, Wf, bf):
+    def forward(ctx, geom, residual, act, s, sbar, v, vbar, W1, b1, W2, b2, Wf, bf, basis, unit):
         s, sbar, v, vbar = s.contiguous(), sbar.contiguous(), v.contiguous(), vbar.contiguous()
         a1, z1, phi = _phi_forward(s, W1, b1, W2, b2, act)
         N, F = s.shape
@@ -145,12 +192,18 @@ class Message9Block(Function):
     @once_differentiable
     def backward(ctx, g_s, g_sbar, g_v, g_vbar):
         s, sbar, v, vbar, a1, z1, phi3, W1, b1, W2, b2, Wf, bf = ctx.saved_tensors
-        gi_s, gi_sbar, gi_v, gi_vbar, g_phi, dWf, dbf = ops.message9_bwd(
-            phi3, s, sbar, v, vbar, ctx.geom, Wf, bf, ctx.residual,
-            g_s.contiguous(), g_sbar.contiguous(), g_v.contiguous(), g_vbar.contiguous())
+        geom_grad = ctx.needs_input_grad[13] or ctx.needs_input_grad[14]
+        g_v = g_v.contiguous()
+        args = (phi3, s, sbar, v, vbar, ctx.geom, Wf, bf, ctx.residual, g_s.contiguous(), g_sbar.contiguous(), g_v,
+                g_vbar.contiguous())
+        outs = ops.message9_bwd(*args, keep_gw=True) if geom_grad else ops.message9_bwd(*args)
+        gi_s, gi_sbar, gi_v, gi_vbar, g_phi, dWf, dbf = outs[:7]
+        d_basis = d_unit = None
+        if geom_grad:
+            d_basis, d_unit = ops.message9_geom_bwd(phi3, ctx.geom, Wf, bf, outs[7], g_v)
         N, F = s.shape
         gs, gW1, gb1, gW2, gb2 = _phi_backward(g_phi.view(N, 9 * F), s, a1, z1, W1, b1, W2, b2, gi_s, ctx.act)
-        return None, None, None, gs, gi_sbar, gi_v, gi_vbar, gW1, gb1, gW2, gb2, dWf, dbf
+        return None, None, None, gs, gi_sbar, gi_v, gi_vbar, gW1, gb1, gW2, gb2, dWf, dbf, d_basis, d_unit
 
 
 class UpdateBlockFn(Function):
@@ -259,7 +312,8 @@ class EmbeddingLookup(Function):
 
 
 class Lift(Function):
-    """bead -> atom lifting (cgvae.py:466-482; PCN cgvae.py:556-576): V [Nc,3,F] -> xyz [N,3]."""
+    """bead -> atom lifting (cgvae.py:466-482; PCN cgvae.py:556-576): V [Nc,3,F] -> xyz [N,3].  Every atom is its bead's
+    position plus an offset, in all three modes, so the gradient to cg_xyz is the per-bead sum of the atom gradients."""
 
     @staticmethod
     def forward(ctx, seg, mode, pin, V, cg_xyz):
@@ -269,7 +323,9 @@ class Lift(Function):
     @staticmethod
     @once_differentiable
     def backward(ctx, g):
-        return None, None, None, ops.lift_bwd(g.contiguous(), ctx.seg, ctx.F, ctx.mode, ctx.pin), None
+        g = g.contiguous()
+        g_cg = ops.segment_reduce_fwd(g, ctx.seg, False) if ctx.needs_input_grad[4] else None
+        return None, None, None, ops.lift_bwd(g, ctx.seg, ctx.F, ctx.mode, ctx.pin), g_cg
 
 
 class VAELatent(Function):
@@ -310,7 +366,9 @@ class StdLogvar(Function):
 
 class TrainingLoss(Function):
     """scripts/utils.py:117-141 as one node: returns (loss [1], components [4] = loss, recon, kl, graph; not differentiable).
-    Gradients flow to xyz_recon, mu, sigma and the prior mean / std; the bond term uses the CSR of the symmetrised bond list."""
+    Gradients flow to xyz_recon, mu, sigma and the prior mean / std, and to the target xyz when it requires grad (the
+    encoder input of a CGequiVAE batch whose coordinates are differentiated); the bond term uses the CSR of the symmetrised
+    bond list."""
 
     @staticmethod
     def forward(ctx, bond_graph, beta, gamma, norms, xyz, xyz_rec, mu, sigma, pmu, pstd):
@@ -342,7 +400,8 @@ class TrainingLoss(Function):
         g = g_loss.reshape(1).contiguous()
         g_rec, g_mu, g_sigma, g_pmu, g_pstd = ops.loss_bwd(g, xyz, xyz_rec, ctx.bond_graph, mu, sigma, pmu, pstd, ctx.norms,
                                                            ctx.beta, ctx.gamma)
-        return None, None, None, None, None, g_rec, g_mu, g_sigma, g_pmu, g_pstd
+        g_xyz = ops.loss_bwd_target(g, xyz, xyz_rec, ctx.bond_graph, ctx.norms, ctx.gamma) if ctx.needs_input_grad[4] else None
+        return None, None, None, None, g_xyz, g_rec, g_mu, g_sigma, g_pmu, g_pstd
 
 
 class DihedralLoss(Function):
@@ -365,6 +424,8 @@ class DihedralLoss(Function):
     @staticmethod
     @once_differentiable
     def backward(ctx, g):
+        if ctx.needs_input_grad[0]:
+            raise NotImplementedError("coordinate gradients: the gradient of the dihedral loss to its target xyz is not implemented")
         (contrib,) = ctx.saved_tensors
         g_rec = ops.dihedral_loss_bwd(g.reshape(1).contiguous(), contrib, ctx.graph, ctx.n_atoms, ctx.count, ctx.norm)
         return None, g_rec, None, None, None

@@ -405,6 +405,39 @@ def edge_geometry(graph, xyz_send, xyz_recv, n_rbf, cutoff, edge_wgt=None, r_edg
     return Geometry(graph, basis, unit, n_rbf, rb, cutoff)
 
 
+def edge_geometry_bwd(graph, n_rbf, cutoff, xyz_send, xyz_recv, d_basis, d_unit, edge_wgt=None, r_edge=None):
+    """cotangent of the edge displacements from those of the basis / unit records of edge_geometry (either may be None =
+    zero): [E,3] in receiver-CSR slot order, or, with r_edge, the gradient of r_edge in its original edge order."""
+    _need_cuda(xyz_send, xyz_recv, r_edge)
+    lib = _lib.load()
+    g = graph
+    E = g.n_edges
+    dev = g.rowptr.device
+    coef = rbf_coefficients(n_rbf, cutoff, dev)
+    dr = torch.empty((E, 3), dtype=torch.float32, device=dev)
+    xs = _f32(xyz_send) if xyz_send is not None else None
+    xr = _f32(xyz_recv) if xyz_recv is not None else None
+    re = _f32(r_edge) if r_edge is not None else None
+    w = _f32(edge_wgt) if edge_wgt is not None else None
+    db = _f32(d_basis) if d_basis is not None else None
+    du = _f32(d_unit) if d_unit is not None else None
+    _lib.check(lib.cgvae_edge_geometry_bwd(_p(xs), _p(xr), _p(re), _p(g.rowptr), _p(g.col), g.n_recv, E, _p(coef), n_rbf, rb_for(n_rbf),
+                                           float(np.float32(cutoff)), _p(w), _p(g.eid), _p(db), _p(du), _p(dr), _stream()),
+               "edge_geometry_bwd")
+    return dr
+
+
+def edge_coord_reduce(graph, dr, same):
+    """(g_send [n_send,3], g_recv [n_recv,3] or None when ``same``) from per-slot displacement cotangents dr."""
+    _need_cuda(dr)
+    lib = _lib.load()
+    g_send = torch.empty((graph.n_send, 3), dtype=torch.float32, device=dr.device)
+    g_recv = None if same else torch.empty((graph.n_recv, 3), dtype=torch.float32, device=dr.device)
+    _lib.check(lib.cgvae_edge_coord_reduce(_p(dr), _p(graph.rowptr), graph.n_recv, _p(graph.rowptr_t), _p(graph.perm_t), graph.n_send,
+                                           int(bool(same)), _p(g_send), _p(g_recv), _stream()), "edge_coord_reduce")
+    return g_send, g_recv
+
+
 # --------------------------------------------------------------------------------------------------
 # dense
 # --------------------------------------------------------------------------------------------------
@@ -804,6 +837,35 @@ def message_bwd(n_split, phi, v_send, v_recv, q, geom, Wf, bf, g_out_s, g_out_v,
     return g_phi, g_v, dWf, dbf
 
 
+def message_geom_bwd(n_split, phi, v_send, v_recv, geom, Wf, bf, g_out_s, g_out_v):
+    """geometry cotangents of one message layer: (d_basis [E,RB], d_unit [E,4]); n_split 9 returns (None, d_unit)."""
+    _need_cuda(phi)
+    lib = _lib.load()
+    g = geom.graph
+    F = phi.shape[-1]
+    dev = phi.device
+    d_basis = torch.empty((g.n_edges, geom.rb), dtype=torch.float32, device=dev) if n_split != 9 else None
+    d_unit = torch.empty((g.n_edges, 4), dtype=torch.float32, device=dev)
+    _lib.check(lib.cgvae_message_geom_bwd(n_split, _p(phi), _p(v_send), _p(v_recv), _p(g.rowptr), _p(g.col), g.n_recv, g.n_edges,
+                                          _p(geom.basis), _p(geom.unit), _p(Wf), _p(bf), F, geom.n_rbf, geom.rb, _p(g_out_s),
+                                          _p(g_out_v), int(v_send is None), _p(d_basis), _p(d_unit), _stream()), "message_geom_bwd")
+    return d_basis, d_unit
+
+
+def message9_geom_bwd(phi, geom, Wf, bf, gw, g_v):
+    """geometry cotangents of a 9-split layer: d_basis = gw [Wf | bf] with cgvae_gemm (gw from message9_bwd, padded
+    basis columns zero), d_unit from the unit-only form of cgvae_message_geom_bwd."""
+    g = geom.graph
+    E, R, F = g.n_edges, geom.n_rbf, phi.shape[-1]
+    d_basis = fill((E, geom.rb), 0.0, phi)
+    if E > 0:
+        with matmul_precision("highest"):           # fp32 in both precision modes, like every coordinate-gradient kernel
+            gemm(GEMM_NN, gw, Wf, E, R, 9 * F, out=d_basis[:, :R])
+            gemm(GEMM_NN, gw, bf.view(9 * F, 1), E, 1, 9 * F, out=d_basis[:, R:R + 1])
+    _, d_unit = message_geom_bwd(9, phi, None, None, geom, Wf, bf, None, g_v)
+    return d_basis, d_unit
+
+
 def message9_fwd(phi, s, sbar, v, vbar, geom, Wf, bf, residual):
     _need_cuda(phi)
     lib = _lib.load()
@@ -816,8 +878,8 @@ def message9_fwd(phi, s, sbar, v, vbar, geom, Wf, bf, residual):
     return outs
 
 
-def message9_bwd(phi, s, sbar, v, vbar, geom, Wf, bf, residual, g_s, g_sbar, g_v, g_vbar):
-    """returns (gi_s, gi_sbar, gi_v, gi_vbar, g_phi [n,9,F], dWf [9F,R], dbf [9F])."""
+def message9_bwd(phi, s, sbar, v, vbar, geom, Wf, bf, residual, g_s, g_sbar, g_v, g_vbar, keep_gw=False):
+    """returns (gi_s, gi_sbar, gi_v, gi_vbar, g_phi [n,9,F], dWf [9F,R], dbf [9F]), and gw [E,9F] last with keep_gw."""
     _need_cuda(phi)
     lib = _lib.load()
     g = geom.graph
@@ -848,6 +910,8 @@ def message9_bwd(phi, s, sbar, v, vbar, geom, Wf, bf, residual, g_s, g_sbar, g_v
     else:
         dWf = torch.zeros((9 * F, R), dtype=torch.float32, device=dev)
         dbf = torch.zeros((9 * F,), dtype=torch.float32, device=dev)
+    if keep_gw:
+        return gi[0], gi[1], gi[2], gi[3], g_phi, dWf, dbf, gw
     return gi[0], gi[1], gi[2], gi[3], g_phi, dWf, dbf
 
 
@@ -1159,6 +1223,17 @@ def loss_bwd(g_loss, xyz, xyz_rec, bond_graph, mu, sigma, pmu, pstd, norms, beta
                                   F, _p(norms), float(beta), float(gamma), _p(g_rec), _p(g_mu), _p(g_sigma), _p(g_pmu), _p(g_pstd),
                                   _stream()), "loss_bwd")
     return g_rec, g_mu, g_sigma, g_pmu, g_pstd
+
+
+def loss_bwd_target(g_loss, xyz, xyz_rec, bond_graph, norms, gamma):
+    """gradient of the training loss to its target coordinates xyz [n_atoms,3]"""
+    lib = _lib.load()
+    g_xyz = torch.empty_like(xyz)
+    _lib.check(lib.cgvae_loss_bwd_target(_p(g_loss), _p(xyz), _p(xyz_rec), xyz.shape[0],
+                                         _p(bond_graph.rowptr) if bond_graph is not None else None,
+                                         _p(bond_graph.col) if bond_graph is not None else None, _p(norms), float(gamma), _p(g_xyz),
+                                         _stream()), "loss_bwd_target")
+    return g_xyz
 
 
 def pin_mask(idx, n_atoms, count=None):

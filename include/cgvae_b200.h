@@ -129,6 +129,21 @@ int cgvae_edge_geometry(const float* xyz_send, const float* xyz_recv, const floa
                         const float* edge_wgt, const int32_t* eid, float* basis, float* unit,
                         cgvae_stream_t stream);
 
+/* Backward of cgvae_edge_geometry (the reference's autograd of conv.py:25-29, modules.py:52-58,148-172): per-edge
+ * displacement cotangent dr from the cotangents d_basis[E][RB] and d_unit[E][4] (either nullable = zero), same arguments
+ * as the forward.  Without r_edge: dr[E][3] in receiver-CSR slot order; with r_edge: dr[eid[e]] in ORIGINAL edge order
+ * (the gradient of r_edge).  Padded tail slots of a static-capacity graph give zero.  Deterministic. */
+int cgvae_edge_geometry_bwd(const float* xyz_send, const float* xyz_recv, const float* r_edge, const int32_t* rowptr,
+                            const int32_t* col, int64_t n_recv, int64_t n_edges, const float* coef, int R, int RB, float cutoff,
+                            const float* edge_wgt, const int32_t* eid, const float* d_basis, const float* d_unit, float* dr,
+                            cgvae_stream_t stream);
+/* Coordinate gradients from dr[E][3] (receiver-CSR order, r_e = x_send[j] - x_recv[i]): g_send[n_send][3] = sum over the
+ * sender CSR (rowptr_t, perm_t), g_recv[n_recv][3] = -sum over the receiver CSR, each in CSR order.  same != 0: sender and
+ * receiver are one coordinate tensor, g_send = both terms, g_recv unused. */
+int cgvae_edge_coord_reduce(const float* dr, const int32_t* rowptr, int64_t n_recv, const int32_t* rowptr_t,
+                            const int32_t* perm_t, int64_t n_send, int same, float* g_send, float* g_recv,
+                            cgvae_stream_t stream);
+
 /* ------------------------------------------------------------------ dense contractions */
 
 /* Dense / nn.Linear forward and backward contractions (modules.py:75-114, conv.py:41-49,568-586).
@@ -199,6 +214,19 @@ int cgvae_message_bwd(int n_split, const float* phi, const float* v_send, const 
                       const float* g_out_s, const float* g_out_v, int residual, int v_is_zero,
                       float* g_phi, float* g_v_send, float* dWf, float* dbf,
                       void* ws, size_t ws_bytes, cgvae_stream_t stream);
+
+/* Geometry cotangents of a message layer (csrc/message_geom.cu), run only when a coordinate requires grad.  Receiver-CSR
+ * slot order, one store per edge, fixed summation order; same operands as cgvae_message_fwd plus the layer's output
+ * gradients g_out_s[n_recv][F], g_out_v[n_recv][3][F].
+ *   n_split 3, 4: d_basis[E][RB] = sum_k,f gm_k phi_j[k] Wf'[kF+f][.] with gm = (<g_v,v_j>, g_s, <g_v,u>, <g_v,v_i x v_j>),
+ *                 d_unit[E][4] = (sum_f phi_j[2] w[2] g_v[c], 0)
+ *   n_split 9:    unit-only form: d_unit from split 1 (EquiMessagePsuedo); d_basis and g_out_s unused (the caller forms
+ *                 d_basis = gw Wf' from cgvae_message9_bwd's gw with cgvae_gemm).
+ * Padded tail slots get zero. */
+int cgvae_message_geom_bwd(int n_split, const float* phi, const float* v_send, const float* v_recv, const int32_t* rowptr,
+                           const int32_t* col, int64_t n_recv, int64_t n_edges, const float* basis, const float* unit,
+                           const float* Wf, const float* bf, int F, int R, int RB, const float* g_out_s, const float* g_out_v,
+                           int v_is_zero, float* d_basis, float* d_unit, cgvae_stream_t stream);
 
 /* ---- the same layers on the 5th-generation tensor cores (csrc/message_tc.cu) ----
  * Column tiles of a CSR: rows are taken RC (4, 8 or 16) at a time; the columns of a chunk are (sorted union of the partner
@@ -339,6 +367,11 @@ int cgvae_loss_bwd(const float* g_loss, const float* xyz, const float* xyz_rec, 
                    const int32_t* bond_col, const float* mu, const float* sigma, const float* pmu, const float* pstd,
                    int64_t n_beads, int F, const float* norms, float beta, float gamma, float* g_xyz_rec, float* g_mu,
                    float* g_sigma, float* g_pmu, float* g_pstd, cgvae_stream_t stream);
+/* Gradient of the same loss to the TARGET coordinates xyz (needed when xyz is also differentiated as the encoder input):
+ * minus the reconstruction term's gradient plus the bond term's gradient to the target distances |x_a - x_b|_e, gathered
+ * over the same symmetrised bond CSR with the same norms.  g_xyz[n_atoms][3].  One launch, deterministic. */
+int cgvae_loss_bwd_target(const float* g_loss, const float* xyz, const float* xyz_rec, int64_t n_atoms, const int32_t* bond_rowptr,
+                          const int32_t* bond_col, const float* norms, float gamma, float* g_xyz, cgvae_stream_t stream);
 /* Dihedral loss of the PCN loop (scripts/pcn_utils.py:114-132 compute_dihe, :178-180):
  *   out[0] = mean_d (theta(xyz_rec; idx[d]) - theta(xyz; idx[d]))^2,  theta = atan(p1 / (p2 + 1e-6)) exactly as the reference
  * forms it (b1..b3, c1 = b2 x b3, c2 = b1 x b2, p1 = (b1.c1) sqrt(b2.b2 + 1e-6), p2 = c1.c2).  idx int64 [n_dihe][4];
