@@ -9,7 +9,7 @@ from .cgvae import (BatchGraphs, CGequiVAE, CGprior, EquiEncoder, EquivariantDec
                     EquivariantPsuedoDecoder, PCN)
 from .conv import (ContractiveMessageBlock, EquiMessageBlock, EquiMessageCross, EquiMessagePsuedo,  # noqa: F401
                    InvariantMessage, PseudoUpdateBlock, UpdateBlock)
-from .data import (CG_collate, CGDataset, DeviceCGDataset, batch_to, get_neighbor_list,  # noqa: F401
+from .data import (CG_collate, CGDataset, DeviceCGDataset, DeviceProteinDataset, batch_to, get_neighbor_list,  # noqa: F401
                    get_neighbor_list_batch)
 from .modules import Dense, DistanceEmbed, make_directed  # noqa: F401
 from .ops import get_matmul_precision, matmul_precision, set_matmul_precision  # noqa: F401

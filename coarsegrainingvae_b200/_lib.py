@@ -95,6 +95,8 @@ SIGNATURES = {
     "cgvae_fill": (_INT, [_P, _I64, _F32, _P]),
     "cgvae_vec_to_planar": (_INT, [_P, _I64, _INT, _P, _P]),
     "cgvae_vec_from_planar": (_INT, [_P, _I64, _INT, _P, _P]),
+    "cgvae_collate_plan_bytes": (_SZ, []),
+    "cgvae_collate": (_INT, [_P, _P]),
 }
 
 

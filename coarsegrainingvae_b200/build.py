@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libcgvae_sm100.so")
-SOURCES = ["graph.cu", "geom.cu", "gemm.cu", "gemm_tc.cu", "gemm_stream.cu", "message.cu", "message_tc.cu", "message_geom.cu", "nodewise.cu", "loss.cu", "metrics.cu", "optim.cu", "wgrad.cu"]
+SOURCES = ["graph.cu", "geom.cu", "gemm.cu", "gemm_tc.cu", "gemm_stream.cu", "message.cu", "message_tc.cu", "message_geom.cu", "nodewise.cu", "loss.cu", "metrics.cu", "optim.cu", "wgrad.cu", "collate.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=default"]
 

@@ -202,3 +202,180 @@ def CG_collate(dicts):
         else:
             batch[key] = torch.stack([torch.as_tensor(s[key]) for s in shifted], dim=0)
     return batch
+
+
+# Kinds of rows of a protein item (CGVAE_COLLATE_* of the C ABI) and the per-protein arrays they count.
+PROTEIN_KINDS = ("atoms", "residues", "bonds", "ca_edges", "dihedrals", "ca_idx")
+# batch key -> (kind, row width (0: a vector), dtype, kind whose running count the collate adds, or None)
+_PROTEIN_KEYS = (("xyz", 0, 3, torch.float32, None), ("ca_xyz", 1, 3, torch.float32, None), ("res", 1, 0, torch.int64, None),
+                 ("cg_map", 0, 0, torch.int64, 1), ("bond_edge_list", 2, 2, torch.int64, 0),
+                 ("CG_nbr_list", 3, 2, torch.int64, 1), ("ca_idx", 5, 0, torch.int64, 0), ("dihe_idxs", 4, 4, torch.int64, 0))
+# live-count key of every kind in a static batch (train.to_static_pcn_batch names, plus atom_count / res_count)
+_PROTEIN_COUNT_KEYS = ("atom_count", "res_count", "bond_count", "CG_nbr_count", "dihe_count", "ca_count")
+# the capacity of a kind is the row count of this key ("ca_xyz" rows include the pad beads)
+_PROTEIN_CAP_KEYS = ("xyz", "ca_xyz", "bond_edge_list", "CG_nbr_list", "dihe_idxs", "ca_idx")
+
+
+def protein_capacities(sizes, atoms_per_bead, batch_size=None, batches=None):
+    """Static capacities of a protein batch from a size table ``sizes [P, 6]`` (columns in ``PROTEIN_KINDS`` order),
+    keyed like the batch tensors whose row count they fix.  Default: per kind, the sum of the ``batch_size`` largest
+    entries.  ``batches`` (planned lists of item indices, -1 = empty slot): per kind, the largest total over those batches.
+    ``ca_xyz`` adds ceil(atoms / atoms_per_bead) pad beads, so the pad atoms of a batch can be spread over beads of at most
+    ``atoms_per_bead`` atoms each."""
+    sizes = np.asarray(sizes, dtype=np.int64).reshape(-1, len(PROTEIN_KINDS))
+    if batches is not None:
+        tot = np.zeros(len(PROTEIN_KINDS), dtype=np.int64)
+        for b in batches:
+            b = np.asarray(b, dtype=np.int64).reshape(-1)
+            tot = np.maximum(tot, sizes[b[b >= 0]].sum(0))
+    elif batch_size is not None:
+        tot = -np.sort(-sizes, axis=0)[:int(batch_size)].sum(0)
+    else:
+        raise ValueError("protein_capacities needs batch_size or batches")
+    caps = {key: int(t) for key, t in zip(_PROTEIN_CAP_KEYS, tot)}
+    caps["ca_xyz"] += -(-caps["xyz"] // int(atoms_per_bead))
+    return caps
+
+
+class DeviceProteinDataset(object):
+    """HBM-resident protein set of the protein-completion path (``SCNCGDataset`` + ``SCNCG_collate``, data.py:292-398 of the
+    reference) for proteins of different lengths.
+
+    ``proteins``: a list of per-protein dicts in the reference's item layout with frame-local indices -- ``xyz [n_at,3]``,
+    ``ca_xyz [n_res,3]``, ``res [n_res]``, ``cg_map [n_at]`` (residue of each atom), ``bond_edge_list [n_b,2]``,
+    ``dihe_idxs [n_d,4]`` and ``ca_idx [n_c]`` (atom indices), optional ``seq``.  Every array goes into one concatenated
+    device store per kind of row with an int64 row-offset table.  The C-alpha graph (``get_neighbor_list(ca_xyz, cg_cutoff,
+    True)`` of data.py:357) is built once, for all proteins in one batched launch, and stored the same way: the coordinates
+    never change, so the collate is a pure gather.
+
+    ``collate(idx)`` returns the dict the host pipeline builds (per-protein dicts concatenated, indices offset by the
+    running atom / residue counts).  ``collate(idx, static=True)`` returns capacity-padded tensors with device live counts
+    for ``GraphedTrainStep``: two launches, no host synchronisation, graph-capturable.  Pads are inert for the PCN: pad
+    atoms have zero coordinates and map, at most ``atoms_per_bead`` to a bead, to pad residues with ``res = 0`` (the
+    embedding's padding row), zero coordinates and no edges, bonds, dihedrals or C-alpha entries."""
+
+    def __init__(self, proteins, cg_cutoff, device='cuda'):
+        dev = torch.device(device)
+        if dev.type != 'cuda':
+            raise RuntimeError("DeviceProteinDataset lives on a CUDA device (device=%r); no CPU fallback" % (device,))
+        self.device, self.cg_cutoff = dev, cg_cutoff
+        P = len(proteins)
+        host = {key: [] for key, *_ in _PROTEIN_KEYS if key != "CG_nbr_list"}
+        sizes = np.zeros((P, len(PROTEIN_KINDS)), dtype=np.int64)
+        self.atoms_per_bead = 1
+        for p, item in enumerate(proteins):
+            arr = {}
+            for key, kind, width, dtype, _ in _PROTEIN_KEYS:
+                if key == "CG_nbr_list":
+                    continue
+                shape = (-1, width) if width else (-1,)
+                val = item.get(key)
+                t = torch.zeros((0, width) if width else (0,), dtype=dtype) if val is None else \
+                    torch.as_tensor(np.asarray(val) if not torch.is_tensor(val) else val).detach().cpu().to(dtype)
+                if t.numel() == 0:
+                    t = t.reshape((0, width) if width else (0,))
+                if tuple(t.shape[1:]) != tuple(shape[1:]) or t.dim() != len(shape):
+                    raise ValueError("protein %d: %s has shape %s, expected [n%s]" % (p, key, tuple(t.shape),
+                                                                                       ", %d" % width if width else ""))
+                arr[key] = t.contiguous()
+            n_at, n_res = int(arr["xyz"].shape[0]), int(arr["ca_xyz"].shape[0])
+            if arr["cg_map"].shape[0] != n_at or arr["res"].shape[0] != n_res:
+                raise ValueError("protein %d: cg_map must have one entry per atom and res one per residue" % p)
+            # every index inside its own protein: a ca_idx entry >= n_atoms would make the pin predicate of cgvae.py:569-571
+            # depend on which proteins share a batch
+            for key, n in (("cg_map", n_res), ("bond_edge_list", n_at), ("dihe_idxs", n_at), ("ca_idx", n_at)):
+                t = arr[key]
+                if t.numel() and (int(t.min()) < 0 or int(t.max()) >= n):
+                    raise IndexError("protein %d: %s entry outside [0, %d)" % (p, key, n))
+            if n_at:
+                self.atoms_per_bead = max(self.atoms_per_bead, int(torch.bincount(arr["cg_map"], minlength=1).max()))
+            for key in host:
+                host[key].append(arr[key])
+            sizes[p] = (n_at, n_res, arr["bond_edge_list"].shape[0], 0, arr["dihe_idxs"].shape[0], arr["ca_idx"].shape[0])
+        self.seq = [item.get("seq") for item in proteins]
+        self.store = {key: torch.cat(v, 0).to(dev).contiguous() if v else None for key, v in host.items()}
+        # C-alpha graph of every protein: one batched launch, split by the residue offsets into frame-local lists
+        res_ptr = torch.zeros(P + 1, dtype=torch.int64)
+        res_ptr[1:] = torch.cumsum(torch.as_tensor(sizes[:, 1]), 0)
+        if P and int(res_ptr[-1]) > 0:
+            pairs = get_neighbor_list_batch(self.store["ca_xyz"], sizes[:, 1], cg_cutoff, True)
+            res_ptr_d = res_ptr.to(dev)
+            owner = torch.searchsorted(res_ptr_d, pairs[:, 0].contiguous(), right=True) - 1
+            self.store["CG_nbr_list"] = (pairs - res_ptr_d[owner][:, None]).contiguous()
+            sizes[:, 3] = torch.bincount(owner, minlength=P).cpu().numpy()
+        else:
+            self.store["CG_nbr_list"] = torch.zeros((0, 2), dtype=torch.int64, device=dev)
+        self.sizes = sizes
+        ptr = np.zeros((len(PROTEIN_KINDS), P + 1), dtype=np.int64)
+        ptr[:, 1:] = np.cumsum(sizes, 0).T
+        self.item_ptr = torch.from_numpy(ptr).to(dev)
+
+    def __len__(self):
+        return len(self.sizes)
+
+    def capacities(self, batch_size=None, batches=None):
+        """``protein_capacities`` of this set's size table (see there)."""
+        return protein_capacities(self.sizes, self.atoms_per_bead, batch_size, batches)
+
+    def _outputs(self, caps):
+        out = {}
+        for key, kind, width, dtype, _ in _PROTEIN_KEYS:
+            rows = caps[_PROTEIN_CAP_KEYS[kind]]
+            out[key] = torch.empty((rows, width) if width else (rows,), dtype=dtype, device=self.device)
+        return out
+
+    def _run(self, idx, out, n_pad_beads, count_out=None, norms=None):
+        outputs, live = [], [0] * len(PROTEIN_KINDS)
+        for key, kind, width, dtype, add in _PROTEIN_KEYS:
+            t = out[key]
+            if t.dtype != dtype or tuple(t.shape[1:]) != ((width,) if width else ()):
+                raise ValueError("%s: expected %s [rows%s], got %s %s" % (key, dtype, ", %d" % width if width else "", t.dtype,
+                                                                        tuple(t.shape)))
+            outputs.append((t, self.store[key], kind, add, key == "cg_map" and n_pad_beads > 0))
+            live[kind] = int(t.shape[0])
+        if out["cg_map"].shape[0] != out["xyz"].shape[0] or out["res"].shape[0] != out["ca_xyz"].shape[0]:
+            raise ValueError("cg_map / xyz and res / ca_xyz must have the same number of rows")
+        live[1] -= n_pad_beads
+        if live[1] < 0:
+            raise ValueError("ca_xyz has fewer rows than the %d pad beads of %d atom rows" % (n_pad_beads, live[0]))
+        return ops.collate(idx, self.item_ptr, outputs, live, self.atoms_per_bead, out["ca_xyz"].shape[0], count_out, norms)
+
+    def _device_idx(self, idx):
+        if torch.is_tensor(idx) and idx.is_cuda:
+            return idx.to(torch.int64).contiguous()
+        t = torch.as_tensor(np.asarray(idx, dtype=np.int64).reshape(-1))
+        return t.pin_memory().to(self.device, non_blocking=True)
+
+    def collate(self, idx, static=False, out=None, capacities=None):
+        """``idx``: item indices (host list / array or int64 tensor on host or device; -1 = empty slot).
+
+        static=False: the unpadded batch of the host pipeline (keys and dtypes of ``synthetic.pcn_batch``; ``seq`` is a
+        list when ``idx`` is on the host).  One host read of the batch size when ``idx`` is on the device.
+
+        static=True: fixed shapes from ``capacities`` (default ``self.capacities(len(idx))``) or from the tensors of ``out``
+        (written in place, e.g. ``GraphedTrainStep.static``), live counts ``atom_count``, ``res_count``, ``bond_count``,
+        ``CG_nbr_count``, ``dihe_count``, ``ca_count`` (int64 [1]) and the loss denominators ``loss_norms`` (float [3]:
+        atoms, residues, bonds) on the device; no host synchronisation.  Inside a CUDA graph capture ``idx`` must be a
+        device tensor.  A batch larger than the capacities is truncated and flagged: ``ops.check_device_errors`` raises."""
+        if not static:
+            idx_h = np.asarray(idx.cpu() if torch.is_tensor(idx) else idx, dtype=np.int64).reshape(-1)
+            if idx_h.size and (idx_h.min() < -1 or idx_h.max() >= len(self)):
+                raise IndexError("protein index outside [-1, %d)" % len(self))
+            tot = self.sizes[idx_h[idx_h >= 0]].sum(0)
+            batch = self._outputs(dict(zip(_PROTEIN_CAP_KEYS, (int(t) for t in tot))))
+            self._run(self._device_idx(idx), batch, 0)
+            if not (torch.is_tensor(idx) and idx.is_cuda):
+                batch = {k: batch[k] for k in ("xyz", "ca_xyz", "res", "cg_map", "bond_edge_list", "CG_nbr_list")} | \
+                    {"seq": [self.seq[i] for i in idx_h if i >= 0], "ca_idx": batch["ca_idx"], "dihe_idxs": batch["dihe_idxs"]}
+            return batch
+        if out is None:
+            n = int(idx.shape[0]) if torch.is_tensor(idx) else len(np.asarray(idx).reshape(-1))
+            out = self._outputs(capacities if capacities is not None else self.capacities(n))
+            for key in _PROTEIN_COUNT_KEYS:
+                out[key] = torch.empty(1, dtype=torch.int64, device=self.device)
+            out["loss_norms"] = torch.empty(3, dtype=torch.float32, device=self.device)
+        n_pad = -(-int(out["xyz"].shape[0]) // self.atoms_per_bead)
+        self._run(self._device_idx(idx), out, n_pad, [out[k] for k in _PROTEIN_COUNT_KEYS], out["loss_norms"])
+        batch = dict(out)
+        batch["CG_nbr_symmetrize"] = True            # one-directional (j > i) C-alpha lists: the CSR kernels add the flip
+        return batch

@@ -304,7 +304,17 @@ class EmbeddingLookup(Function):
     @once_differentiable
     def backward(ctx, g):
         idx, table = ctx.saved_tensors
-        seg = ops.build_segments(idx, ctx.n_rows)
+        n = idx.numel()
+        if ctx.padding_idx is not None and n > 2048:
+            # the padding row's gradient is discarded: its entries go to spare rows of <= 1024 each, past the table, so that
+            # no row outgrows the 2048-entry shared-memory sort of graph.cu (a capacity-padded protein batch holds
+            # thousands of pad residues); the other rows keep their entries in the same order
+            spare = -(-n // 1024)
+            pos = torch.arange(n, dtype=torch.int64, device=idx.device).remainder_(spare).add_(ctx.n_rows)
+            seg = ops.build_segments(torch.where(idx == ctx.padding_idx, pos, idx), ctx.n_rows + spare)
+            seg = ops.Segments(ctx.n_rows, seg.mapping, seg.rowptr, seg.atoms, seg.slot, seg.rank)
+        else:
+            seg = ops.build_segments(idx, ctx.n_rows)
         gt = ops.segment_reduce_fwd(g.contiguous(), seg, False, param=table)
         if ctx.padding_idx is not None:
             gt[ctx.padding_idx].zero_()
@@ -416,7 +426,10 @@ class DihedralLoss(Function):
         out, contrib = ops.dihedral_loss_fwd(xyz.contiguous(), xyz_rec.contiguous(), idx, count, norm)
         D = idx.shape[0]
         pairs = torch.stack([idx.reshape(-1), torch.arange(4 * D, dtype=torch.int64, device=idx.device)], 1)
-        ctx.graph = ops.build_graph(pairs, n_atoms, n_send=max(4 * D, 1))
+        # a padded list's (0, 0, 0, 0) rows stay out of the CSR: they would pile 4 entries per pad row onto atom 0, and rows
+        # that long fall back to the slow in-place sort of graph.cu (seconds per step at protein-batch capacities)
+        live = None if count is None else (count.reshape(1).to(torch.int64) * 4).clamp_(max=4 * D)
+        ctx.graph = ops.build_graph(pairs, n_atoms, n_send=max(4 * D, 1), n_edges_dev=live)
         ctx.n_atoms, ctx.count, ctx.norm = n_atoms, count, norm
         ctx.save_for_backward(contrib)
         return out.reshape(())

@@ -5,6 +5,7 @@ memory), and launches hand-written sm_100a kernels on the current stream through
 CPU path: a non-CUDA tensor raises.  Layouts: scalars [N,F]; vectors planar [N,3,F]; phi [N,K,F].
 """
 import contextlib as _contextlib
+import ctypes
 
 import numpy as np
 import torch
@@ -58,7 +59,8 @@ _ERR_FLAGS = {}
 _ERR_TEXT = {1: "a bead holds more atoms than feature channels (cg_v[mapping, CG2atomChannel], cgvae.py:473)",
              2: "embedding index out of range (nn.Embedding, cgvae.py:273,380,591)",
              4: "CG_mapping entry outside [0, n_beads)",
-             8: "edge-list entry outside [0, n_nodes)"}
+             8: "edge-list entry outside [0, n_nodes)",
+             16: "a collated batch exceeds its capacities, or selects an item outside the dataset"}
 
 
 def error_flags(device):
@@ -1269,3 +1271,66 @@ def dihedral_loss_bwd(g_loss, contrib, graph, n_atoms, count=None, norm=None):
     _lib.check(lib.cgvae_dihedral_loss_bwd(_p(g_loss), _p(contrib), _p(graph.rowptr), _p(graph.col), n_atoms, contrib.shape[0],
                                            _p(count), _p(norm), _p(g), _stream()), "dihedral_loss_bwd")
     return g
+
+
+# --------------------------------------------------------------------------------------------------
+# ragged batch collation (csrc/collate.cu)
+# --------------------------------------------------------------------------------------------------
+
+COLLATE_KINDS = 6          # atoms, residues, bonds, C-alpha edges, dihedrals, C-alpha indices (CGVAE_COLLATE_*)
+COLLATE_MAX_OUT = 8
+
+
+class _CollateOut(ctypes.Structure):
+    _fields_ = [("dst", ctypes.c_void_p), ("src", ctypes.c_void_p), ("rows", ctypes.c_int64), ("width", ctypes.c_int32),
+                ("elem_bytes", ctypes.c_int32), ("kind", ctypes.c_int32), ("add_kind", ctypes.c_int32),
+                ("pad_beads", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
+class CollatePlan(ctypes.Structure):
+    """struct cgvae_collate_plan of include/cgvae_b200.h."""
+    _fields_ = [("idx", ctypes.c_void_p), ("item_ptr", ctypes.c_void_p), ("slot_off", ctypes.c_void_p),
+                ("counts", ctypes.c_void_p), ("count_out", ctypes.c_void_p * COLLATE_KINDS), ("norms", ctypes.c_void_p),
+                ("n_slots", ctypes.c_int64), ("n_items", ctypes.c_int64), ("atoms_per_bead", ctypes.c_int64),
+                ("n_beads", ctypes.c_int64), ("live_cap", ctypes.c_int64 * COLLATE_KINDS), ("n_out", ctypes.c_int32),
+                ("reserved", ctypes.c_int32), ("out", _CollateOut * COLLATE_MAX_OUT)]
+
+
+def collate(idx, item_ptr, outputs, live_cap, atoms_per_bead=1, n_beads=0, count_out=None, norms=None):
+    """cgvae_collate: gather the rows of the items ``idx`` (int64 [B] CUDA, -1 = empty slot) from ragged stores into
+    fixed-size outputs.  item_ptr: int64 [KINDS, n_items+1] CUDA row offsets of every item in every kind's store.
+    outputs: list of (dst, src, kind, add_kind or None, pad_beads) with dst [rows] / [rows, width] and src the kind's store
+    of the same dtype and width.  live_cap: KINDS ints.  count_out: KINDS int64 [1] tensors or None; norms: float [3] or None.
+    Returns the live counts (int64 [KINDS], CUDA).  Two launches, no host synchronisation."""
+    _need_cuda(idx, item_ptr)
+    lib = _lib.load()
+    dev = idx.device
+    if idx.dtype != torch.int64 or not idx.is_contiguous() or not item_ptr.is_contiguous():
+        raise ValueError("collate: idx / item_ptr must be contiguous int64")
+    B = idx.shape[0]
+    slot_off = torch.empty(COLLATE_KINDS * (B + 1), dtype=torch.int64, device=dev)
+    counts = torch.empty(COLLATE_KINDS, dtype=torch.int64, device=dev)
+    plan = CollatePlan()
+    plan.idx, plan.item_ptr, plan.slot_off, plan.counts = _p(idx), _p(item_ptr), _p(slot_off), _p(counts)
+    for k, t in enumerate(count_out or ()):
+        plan.count_out[k] = _p(t)
+    plan.norms = _p(norms)
+    plan.n_slots, plan.n_items = B, item_ptr.shape[1] - 1
+    plan.atoms_per_bead, plan.n_beads = int(atoms_per_bead), int(n_beads)
+    for k, c in enumerate(live_cap):
+        plan.live_cap[k] = int(c)
+    if len(outputs) > COLLATE_MAX_OUT:
+        raise ValueError("collate: at most %d outputs" % COLLATE_MAX_OUT)
+    plan.n_out = len(outputs)
+    for i, (dst, src, kind, add_kind, pad_beads) in enumerate(outputs):
+        _need_cuda(dst, src)
+        width = dst.shape[1] if dst.dim() == 2 else 1
+        if not (dst.is_contiguous() and src.is_contiguous()) or dst.dtype != src.dtype or \
+                (src.shape[1] if src.dim() == 2 else 1) != width or dst.dtype not in (torch.float32, torch.int64):
+            raise ValueError("collate: output %d: dst / src must be contiguous float32 or int64 of the same width" % i)
+        o = plan.out[i]
+        o.dst, o.src, o.rows, o.width, o.elem_bytes = _p(dst), _p(src), dst.shape[0], width, dst.element_size()
+        o.kind, o.add_kind, o.pad_beads = int(kind), -1 if add_kind is None else int(add_kind), int(bool(pad_beads))
+    error_flags(dev)
+    _lib.check(lib.cgvae_collate(ctypes.byref(plan), _stream()), "collate")
+    return counts

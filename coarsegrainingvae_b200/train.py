@@ -227,6 +227,8 @@ class TrainStep(object):
         world = self._world()
         if world == 1:
             return batch
+        if "atom_count" in batch:
+            return self._update_dp_norms_live(batch, world)
         xyz = batch["nxyz"] if "nxyz" in batch else batch["xyz"]
         beads = batch["CG_nxyz"] if "CG_nxyz" in batch else batch["ca_xyz"]
         dev = xyz.device
@@ -239,6 +241,22 @@ class TrainStep(object):
             batch["dp_norms"].copy_(counts)
         else:
             batch["dp_norms"] = counts
+        return batch
+
+    def _update_dp_norms_live(self, batch, world):
+        """capacity-padded batches (data.DeviceProteinDataset.collate(static=True)): all-reduce the LIVE counts (atoms,
+        residues, bonds, dihedrals) on the device; ``dihe_norm`` (device float [1]) gets the global dihedral count / world,
+        so that the dihedral term too is the mean over the global batch and not a mean of per-rank means."""
+        import torch.distributed as dist
+        dihe = batch["dihe_count"] if "dihe_count" in batch else torch.zeros_like(batch["atom_count"])
+        counts = torch.cat([batch["atom_count"], batch["res_count"], batch["bond_count"], dihe]).to(torch.float32)
+        dist.all_reduce(counts, op=dist.ReduceOp.SUM, group=self.group)
+        counts = (counts / world).clamp_min(1.0)
+        for key, val in (("dp_norms", counts[:3]), ("dihe_norm", counts[3:])):
+            if key in batch:
+                batch[key].copy_(val)
+            else:
+                batch[key] = val.clone()
         return batch
 
     def prepare(self, batch, eps=None):
@@ -562,6 +580,8 @@ class PCNTrainStep(TrainStep):
     def _loss(self, batch, eps):
         out = self.model(batch)
         norms = batch.get("dp_norms")
+        if norms is None and "atom_count" in batch:
+            norms = batch["loss_norms"]          # capacity-padded batch: live (atoms, residues, bonds), not the padded shapes
         loss = training_loss(out, out[4], batch["bond_edge_list"], 0.0, self.gamma, batch.get("bond_count"), norms)[0]
         if self.kappa != 0.0 and "dihe_idxs" in batch:
             loss = loss + self.kappa * dihedral_loss(out[5], out[4], batch["dihe_idxs"], batch.get("dihe_count"),
@@ -693,7 +713,7 @@ class GraphedTrainStep(object):
         out = torch.zeros(self.packed.numel(), dtype=torch.uint8, pin_memory=pin) if device is None else \
             torch.zeros(self.packed.numel(), dtype=torch.uint8, device=device)
         for k, o, nbytes, dtype, shape in self.layout:
-            if k == "dp_norms" and k not in batch:      # filled on the device by update_dp_norms before every replay
+            if k in ("dp_norms", "dihe_norm") and k not in batch:    # filled on the device by update_dp_norms before every replay
                 continue
             v = batch[k]
             if tuple(v.shape) != shape or v.dtype != dtype:

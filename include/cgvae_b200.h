@@ -60,7 +60,8 @@ unsigned long long cgvae_launch_count(void);
 enum { CGVAE_ERR_LIFT_RANK_BIT = 1,   /* a bead holds more atoms than channels F (cgvae.py:473) */
        CGVAE_ERR_EMBED_INDEX_BIT = 2, /* embedding id outside the table (cgvae.py:273,380,591) */
        CGVAE_ERR_BEAD_INDEX_BIT = 4,  /* CG_mapping entry outside [0, n_beads) */
-       CGVAE_ERR_NODE_INDEX_BIT = 8   /* edge-list entry outside [0, n_nodes) */ };
+       CGVAE_ERR_NODE_INDEX_BIT = 8,  /* edge-list entry outside [0, n_nodes) */
+       CGVAE_ERR_COLLATE_BIT = 16     /* a collated batch exceeds its capacities, or selects an item outside the set */ };
 int cgvae_set_error_flags(int device, int32_t* flags);
 
 /* ------------------------------------------------------------------ graph builders (integer) */
@@ -387,6 +388,43 @@ int cgvae_dihedral_loss_bwd(const float* g_loss, const float* contrib, const int
  * pin[idx[i]] = 1 for the live entries iff idx[last] < n_atoms.  pin_bytes >= n_atoms, a multiple of 4. */
 int cgvae_pin_mask(const int64_t* idx, int64_t n_idx, const int64_t* n_live, int64_t n_atoms, uint8_t* pin, size_t pin_bytes,
                    cgvae_stream_t stream);
+/* ------------------------------------------------------------------ ragged batch collation
+
+ * SCNCGDataset.__getitem__ + SCNCG_collate (data.py:292-398) for a protein set resident in device memory
+ * (data.DeviceProteinDataset).  Each kind of row has one concatenated store (rows of item p: item_ptr[kind][p] ..
+ * item_ptr[kind][p+1]); idx[n_slots] selects the items of a batch, -1 = empty slot.  One output per stored array:
+ * rows [0, live) = the selected items' rows concatenated in slot order, each int64 row plus the running count of kind
+ * add_kind of the slots before it (the collate offsets); rows [live, rows) = pad: zero, or with pad_beads the pad bead
+ * counts[RESIDUES] + k / atoms_per_bead of pad row k (clamped to n_beads - 1).  counts[kind] = min(total, live_cap[kind]);
+ * a larger total, or an idx entry outside [-1, n_items), sets CGVAE_ERR_COLLATE_BIT and writes nothing past any `rows`.
+ * count_out[kind] (each nullable) receive copies of counts; norms (nullable float[3]) = max(1, counts) of (atoms,
+ * residues, bonds): the loss denominators.  slot_off: workspace [KINDS][n_slots+1] (the per-slot output offsets).
+ * `plan` is a HOST struct (it travels in the kernel parameters); the pointers inside are device pointers.  Two
+ * launches, no host synchronisation, CUDA-graph capturable; integer rows are exact copies. */
+enum { CGVAE_COLLATE_ATOMS = 0, CGVAE_COLLATE_RESIDUES = 1, CGVAE_COLLATE_BONDS = 2, CGVAE_COLLATE_EDGES = 3,
+       CGVAE_COLLATE_DIHEDRALS = 4, CGVAE_COLLATE_CA = 5, CGVAE_COLLATE_KINDS = 6, CGVAE_COLLATE_MAX_OUT = 8 };
+typedef struct cgvae_collate_out {
+  void* dst;                /* [rows][width] */
+  const void* src;          /* store of the output's kind, [item_ptr[kind][n_items]][width] */
+  int64_t rows;             /* capacity rows of dst */
+  int32_t width, elem_bytes; /* elements per row; 4 (float32) or 8 (int64) */
+  int32_t kind, add_kind;   /* count kind of the rows; kind whose running count is added (-1: none) */
+  int32_t pad_beads, reserved;
+} cgvae_collate_out;
+typedef struct cgvae_collate_plan {
+  const int64_t* idx;       /* [n_slots] */
+  const int64_t* item_ptr;  /* [KINDS][n_items+1] */
+  int64_t* slot_off;        /* [KINDS][n_slots+1] workspace */
+  int64_t* counts;          /* [KINDS] */
+  int64_t* count_out[CGVAE_COLLATE_KINDS];
+  float* norms;
+  int64_t n_slots, n_items, atoms_per_bead, n_beads;
+  int64_t live_cap[CGVAE_COLLATE_KINDS];
+  int32_t n_out, reserved;
+  cgvae_collate_out out[CGVAE_COLLATE_MAX_OUT];
+} cgvae_collate_plan;
+size_t cgvae_collate_plan_bytes(void);
+int cgvae_collate(const cgvae_collate_plan* plan, cgvae_stream_t stream);
 /* Sample-quality metrics of the ensemble-sampling loop (scripts/sampling.py:120-194,220-239,324-333).
  * cgvae_bond_graph: bond[i][j] = (i != j) && sqrt(((dx^2+dy^2)+dz^2)) < (radius[i] + radius[j]) * scale, in fp32 and in the
  * reference's operation order (bit-exact adjacency); radius = covalent cutoff radius per atom (COVCUTOFFTABLE, sampling.py:12-118).
